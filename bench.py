@@ -2,7 +2,7 @@
 """Benchmark of the .spz per-gaussian codec hot path (BASELINE.json: encode/decode Mgaussians/s and
 HBM GB/s vs roofline at 1/2/4/8 B200).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--points P] [--sh-degree D]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--points P] [--sh-degree D] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference's own CPU pack/unpack on the host cores
 
@@ -70,7 +70,14 @@ def parse_args():
     ap.add_argument("--cpu-sample-points", type=int, default=0, help="0 = auto")
     ap.add_argument("--traffic-bytes", type=float, default=None,
                     help="dram bytes per launch of the dominant kernel from an ncu --set full capture")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of the last step's encoded and decoded planes to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the B200 arm computed; the reference arm has no outputs to dump")
+    return args
 
 
 def workload_name(n, deg):
@@ -478,6 +485,34 @@ def oracle_block_parity(cloud, packed, decoded, n, deg, frm, to, rank, blocks=6,
     return len(starts), ok, kind
 
 
+DUMP_POINTS = 65536  # 32.5 MB of .npy files at SH degree 3
+
+
+def dump_outputs(out_dir, packed, decoded, n_total, deg, a, b, rank, world):
+    """What encode_device and decode_device returned in the last timed step, for gaussians drawn from the whole
+    cloud with a fixed seed (so every build and every N dumps the same ones): `encoded_<plane>.npy` holds the byte
+    planes and `decoded_<plane>.npy` the float planes, both float32 with one row per gaussian, and `indices.npy`
+    (float64) the global index of each row.  With N > 1 ranks each writes the rows of its shard, as
+    `<name>.rank<r>.npy`."""
+    import numpy as np
+    import torch
+
+    from spz_b200 import codec
+    idx = np.sort(np.random.default_rng(0).choice(n_total, size=min(n_total, DUMP_POINTS), replace=False))
+    idx = idx[(idx >= a) & (idx < b)]
+    rows = torch.from_numpy(idx - a).to(packed.positions.device)
+    arrays = {"indices": idx.astype(np.float64)}
+    for kind, planes, widths in (("encoded", packed.planes(), codec.byte_plane_widths(deg, 3)),
+                                 ("decoded", decoded.planes(), codec.float_plane_widths(deg))):
+        for name, t, w in zip(codec.PLANES, planes, widths):
+            arrays[f"{kind}_{name}"] = (t.view(-1, w)[rows].to(torch.float32).cpu().numpy() if w
+                                        else np.zeros((idx.size, 0), np.float32))
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "" if world == 1 else f".rank{rank}"
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), arr)
+
+
 def link_ceiling(dev, barrier, seconds=1.0, mb=1024):
     """Bare host<->device link of this rank while every other rank does the same: plain pinned
     cudaMemcpyAsync (torch copy_ on pinned tensors), nothing of the codec.  H2D alone, D2H alone, both at
@@ -621,6 +656,8 @@ def run_b200_arm(args):
     launches = ctx.info()["kernel_launches"] - launches0
     enc_ms = statistics.mean(ev[0].elapsed_time(ev[1]) for ev in evs)
     dec_ms = statistics.mean(ev[1].elapsed_time(ev[2]) for ev in evs)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, packed, decoded, n_total, deg, a, b, rank, world)
 
     # ---- parity of what was just timed (outside the timed region) ---------------------------------
     # (1) sampled 64k-point blocks of this rank's shard against the CPU checker; (2) order-sensitive

@@ -31,10 +31,12 @@ def _run_suite(extra_env=None):
     env = dict(os.environ, PYTHONPATH=os.path.join(ROOT, "spz_b200", "pyspz") + os.pathsep + os.environ.get("PYTHONPATH", ""),
                SPZB200_NO_REBUILD="1")
     env.update(extra_env or {})
-    # -c /dev/null + --rootdir: the reference's file runs under no conftest / ini of this repo
+    # -c /dev/null + --rootdir: the reference's file runs under no conftest / ini of this repo.  --confcutdir: without
+    # it pytest takes the ini file's directory (/dev) as the limit and collects down from /, which fails wherever a
+    # directory above the checkout cannot be listed
     return subprocess.run([sys.executable, "-m", "pytest", SUITE, "-q", "-p", "no:cacheprovider", "-c", os.devnull,
-                           "--rootdir", os.path.dirname(SUITE)], capture_output=True, text=True, env=env, timeout=900,
-                          cwd=os.path.dirname(SUITE))
+                           "--rootdir", os.path.dirname(SUITE), "--confcutdir", os.path.dirname(SUITE)],
+                          capture_output=True, text=True, env=env, timeout=900, cwd=os.path.dirname(SUITE))
 
 
 @pytest.mark.gpu
