@@ -251,6 +251,44 @@ int spzb200_gzip(const uint8_t *data, size_t size, int32_t threads, uint8_t **ou
 int spzb200_gunzip(const uint8_t *data, size_t size, int32_t threads, uint8_t **out, size_t *out_size);
 void spzb200_free(void *ptr);
 
+/* ---- .spz files of device-resident clouds ---------------------------------------------------
+ *
+ * The gzip stage on the device: the input is cut into 64 KiB segments, each coded by one CTA as an
+ * independent piece of a raw deflate stream (Huffman-coded literals plus distance-1 matches for runs of
+ * one byte value; stored when that is not larger), and the pieces are framed as ONE standard gzip member
+ * with the block table spzb200_gzip(threads > 1) writes, so any inflater reads it and spzb200_gunzip
+ * inflates it block-parallel.  The bytes depend only on the input bytes (not on the device, context,
+ * stream or timing).  Only compressed bytes cross PCIe.  *out is malloc'd: release it with spzb200_free.
+ * Synchronous: each returns when *out is complete, after work queued earlier on `stream` (a
+ * cudaStream_t, NULL = legacy default stream).  Device scratch, allocated and freed on `stream`:
+ * about 2 bytes per input byte (the 64 KiB + 64 byte worst-case slot of every segment plus the
+ * compacted body). */
+int spzb200_gzip_device(SpzB200Context *ctx, const uint8_t *data /* device */, size_t size, uint8_t **out, size_t *out_size,
+                        void *stream);
+
+/* saveSpz for a device cloud: the encoder's planes, the 16-byte header and the planes in container order
+ * (positions, alphas, colors, scales, rotations, sh) on the device, then spzb200_gzip_device's deflater.
+ * The file inflates to the container saveSpz writes for the same cloud, `from` and antialiased flag.
+ * Device scratch peaks at about twice the container (65 bytes per point at SH degree 3).  A cloud the
+ * reference's checkSizes rejects, or one of more than 2^31 - 1 points, fails with SPZB200_ERR_INVALID;
+ * nothing is written to any file. */
+int spzb200_save_spz_device(SpzB200Context *ctx, const SpzB200Cloud *in /* device */, int32_t from, int32_t antialiased,
+                            uint8_t **out, size_t *out_size, void *stream);
+
+/* Point count and SH degree from the header of an .spz file in host memory (inflates only the first 16
+ * bytes), to size the output of spzb200_load_spz_device. */
+int spzb200_spz_info(const uint8_t *bytes, size_t size, int64_t *num_points, int32_t *sh_degree);
+
+/* loadSpz into caller-allocated DEVICE planes: inflates on the host (block-parallel for members with the
+ * block table, serially for others such as the reference's files), validates the header the way loadSpz
+ * does before anything is allocated, copies each plane to the device and decodes it with the device
+ * decoder (container versions 1-3).  out->num_points and out->sh_degree must be what spzb200_spz_info
+ * reports.  `to` is UnpackOptions::to; *antialiased (may be NULL) receives the header flag.  A file that
+ * does not inflate or parse fails with SPZB200_ERR_INVALID and leaves `out` untouched.  Device scratch:
+ * the packed planes (the container's size).  Returns when `out` is complete. */
+int spzb200_load_spz_device(SpzB200Context *ctx, const uint8_t *bytes /* host */, size_t size, int32_t to,
+                            SpzB200Cloud *out /* device */, int32_t *antialiased, void *stream);
+
 /* Point range [*begin, *end) of shard `index` out of `num_shards` over n gaussians of the given
  * SH degree.  Boundaries are multiples of the kernel tile, so every shard but the last runs
  * entirely on the vector path and every plane slice stays 16-byte aligned. */

@@ -193,6 +193,14 @@ def gunzip_bytes(data, threads: int = 1) -> bytes:
     return _host_bytes_call(N.lib().spzb200_gunzip, data, threads)
 
 
+def spz_info(blob):
+    """(num_points, sh_degree) from the header of .spz bytes (spzb200_spz_info; inflates 16 bytes, no GPU)."""
+    buf = np.frombuffer(blob, np.uint8) if not isinstance(blob, np.ndarray) else np.ascontiguousarray(blob, np.uint8)
+    n, deg = C.c_int64(0), C.c_int32(0)
+    N.check(N.lib().spzb200_spz_info(C.c_void_p(buf.ctypes.data if buf.size else None), buf.size, C.byref(n), C.byref(deg)))
+    return n.value, deg.value
+
+
 def shard_range(n: int, sh_degree: int, num_shards: int, index: int):
     """Contiguous point range of one shard (host logic, no GPU): spzb200_shard_range."""
     a, b = C.c_int64(0), C.c_int64(0)
@@ -322,6 +330,44 @@ class Context:
         ps, cs = _packed_struct(packed, True), _cloud_struct(out, True)
         N.check(N.lib().spzb200_decode_device(self._h, C.byref(ps), int(to), C.byref(cs), C.c_void_p(self._stream_handle(stream))))
         return out
+
+    # ---- .spz files of device-resident clouds (the deflate stage on the device) ------------------
+    def _take_bytes(self, rc: int, out: C.c_void_p, size: C.c_size_t) -> bytes:
+        N.check(rc)
+        try:
+            return C.string_at(out.value, size.value)
+        finally:
+            N.lib().spzb200_free(out)
+
+    def gzip_device(self, data, stream=None) -> bytes:
+        """A contiguous uint8 CUDA tensor -> one gzip member, deflated on the device (spzb200_gzip_device)."""
+        ptr = _ptr(data, "u1", data.numel(), True, "data")
+        out, size = C.c_void_p(None), C.c_size_t(0)
+        rc = N.lib().spzb200_gzip_device(self._h, C.c_void_p(ptr), data.numel(), C.byref(out), C.byref(size),
+                                         C.c_void_p(self._stream_handle(stream)))
+        return self._take_bytes(rc, out, size)
+
+    def save_spz_device(self, cloud: CloudPlanes, frm: int = 0, antialiased: bool = False, stream=None) -> bytes:
+        """The .spz file of a device cloud (spzb200_save_spz_device): what saveSpz writes, inflated."""
+        cs = _cloud_struct(cloud, True)
+        out, size = C.c_void_p(None), C.c_size_t(0)
+        rc = N.lib().spzb200_save_spz_device(self._h, C.byref(cs), int(frm), int(bool(antialiased)), C.byref(out), C.byref(size),
+                                             C.c_void_p(self._stream_handle(stream)))
+        return self._take_bytes(rc, out, size)
+
+    def load_spz_device(self, blob, to: int = 0, device=None, out: Optional[CloudPlanes] = None, stream=None):
+        """.spz bytes -> (CloudPlanes of CUDA tensors, antialiased) via spzb200_load_spz_device.  `out`, if
+        given, must match the file's point count and SH degree (spz_info)."""
+        buf = np.frombuffer(blob, np.uint8) if not isinstance(blob, np.ndarray) else np.ascontiguousarray(blob, np.uint8)
+        if out is None:
+            n, deg = spz_info(buf)
+            out = alloc_cloud(n, deg, device=device if device is not None else f"cuda:{self.device}")
+        cs = _cloud_struct(out, True)
+        aa = C.c_int32(0)
+        N.check(N.lib().spzb200_load_spz_device(self._h, C.c_void_p(buf.ctypes.data if buf.size else None), buf.size, int(to), C.byref(cs),
+                                                C.byref(aa), C.c_void_p(self._stream_handle(stream))))
+        out.antialiased = bool(aa.value)
+        return out, out.antialiased
 
     # ---- fused PLY-rows encoder ---------------------------------------------------------------
     def encode_ply_device(self, rows, n: int, names, sh_degree: int, frm: int = 0, out: Optional[PackedPlanes] = None, stream=None):

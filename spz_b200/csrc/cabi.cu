@@ -7,6 +7,7 @@
 //   * the 255 thresholds of the alpha quantizer  a -> toUint8(sigmoid(a) * 255)   (uses expf)
 //   * the 256 values of the alpha dequantizer    b -> invSigmoid(b / 255.0f)      (uses logf)
 #include <cuda_runtime.h>
+#include <zlib.h>
 #if defined(__x86_64__) && (defined(__GNUC__) || defined(__clang__))
 #include <immintrin.h>
 #endif
@@ -33,6 +34,8 @@
 #include "../../include/spz_b200/spz.hpp"
 #include "codec_kernels.cuh"
 #include "codec_math.cuh"
+#include "deflate_format.cuh"
+#include "spz_internal.hpp"
 
 namespace {
 
@@ -1893,6 +1896,260 @@ int spzb200_unpack_gather_device(SpzB200Context *ctx, const SpzB200Packed *packe
   CU(spzb200::launchUnpackRecords(a, (cudaStream_t)stream, &launches));
   ctx->kernelLaunches += launches;
   return SPZB200_OK;
+}
+
+}  // extern "C"
+
+// =================================================================================================
+// .spz files from and to device-resident planes, with the deflate stage on the device (DESIGN.md section 10)
+// =================================================================================================
+
+namespace {
+
+// Device scratch of one call: stream-ordered allocations, handed back on the same stream on every exit.
+struct DeviceScratch {
+  cudaStream_t stream;
+  std::vector<void *> ptrs;
+  explicit DeviceScratch(cudaStream_t s) : stream(s) {}
+  ~DeviceScratch() {
+    for (void *p : ptrs) cudaFreeAsync(p, stream);
+  }
+  template <class T>
+  cudaError_t alloc(T **p, size_t bytes) {
+    void *v = nullptr;
+    const cudaError_t e = cudaMallocAsync(&v, std::max<size_t>(bytes, 16), stream);
+    if (e != cudaSuccess) return e;
+    ptrs.push_back(v);
+    *p = static_cast<T *>(v);
+    return cudaSuccess;
+  }
+};
+
+size_t deflateBodyBytes(size_t size) { return size + 16 * spzb200::dfl::segmentCount(size) + 16; }
+
+// `size` device bytes at src -> one gzip member in *out.  slots: segmentCount * deflateSlotBytes() bytes; body:
+// deflateBodyBytes(size) bytes (may be src itself: the body is written after the last read of src).  Synchronous.
+int gzipDeviceBytes(SpzB200Context *ctx, const uint8_t *src, size_t size, uint8_t *slots, uint8_t *body, DeviceScratch &scratch,
+                    std::vector<uint8_t> *out) {
+  namespace dfl = spzb200::dfl;
+  const size_t segs = dfl::segmentCount(size);
+  uint32_t *segBytes = nullptr;
+  unsigned long long *offsets = nullptr;
+  CU(scratch.alloc(&segBytes, 2 * segs * sizeof(uint32_t)));
+  CU(scratch.alloc(&offsets, (segs + 1) * sizeof(unsigned long long)));
+  uint32_t *segCrc = segBytes + segs;
+  int launches = 0;
+  CU(spzb200::launchDeflate(src, size, slots, segBytes, segCrc, offsets, body, scratch.stream, &launches));
+  ctx->kernelLaunches += launches;
+  std::vector<uint32_t> hostSeg(2 * segs);
+  CU(cudaMemcpyAsync(hostSeg.data(), segBytes, 2 * segs * sizeof(uint32_t), cudaMemcpyDeviceToHost, scratch.stream));
+  CU(cudaStreamSynchronize(scratch.stream));
+  uLong crc = crc32(0L, Z_NULL, 0);
+  const size_t perBlock = dfl::segmentsPerBlock(segs);
+  std::vector<uint32_t> blockBytes((segs + perBlock - 1) / perBlock, 0);
+  for (size_t s = 0; s < segs; s++) {
+    const size_t len = std::min<size_t>(dfl::kSegBytes, size - std::min(size, s * dfl::kSegBytes));
+    crc = crc32_combine(crc, hostSeg[segs + s], (z_off_t)len);
+    blockBytes[s / perBlock] += hostSeg[s];
+  }
+  // The body comes back in pieces through two of the context's pinned bounce buffers: the DMA of one piece
+  // overlaps the host copy of the previous one (a pageable D2H of the whole body ran at ~2 GB/s on a B200 host).
+  constexpr size_t kPiece = (size_t)8 << 20;
+  int brc = SPZB200_OK;
+  for (int k = 0; k < 2 && brc == SPZB200_OK; k++) brc = ensureBounce(ctx->stage[k].hOut, ctx->stage[k].hOutCap, kPiece);
+  if (brc) return brc;
+  cudaError_t copy = cudaSuccess;
+  const bool ok = spz::detail::frameBlockMember(size, perBlock * dfl::kSegBytes, blockBytes, (uint32_t)crc,
+                                                [&](uint8_t *dst) {
+                                                  size_t total = 0;
+                                                  for (uint32_t b : blockBytes) total += b;
+                                                  const size_t pieces = (total + kPiece - 1) / kPiece;
+                                                  auto len = [&](size_t i) { return std::min(kPiece, total - i * kPiece); };
+                                                  for (size_t i = 0; i <= pieces && copy == cudaSuccess; i++) {
+                                                    if (i < pieces) {
+                                                      Stage &s = ctx->stage[i & 1];
+                                                      copy = cudaMemcpyAsync(s.hOut, body + i * kPiece, len(i), cudaMemcpyDeviceToHost, scratch.stream);
+                                                      if (copy == cudaSuccess) copy = cudaEventRecord(s.ev[0], scratch.stream);
+                                                    }
+                                                    if (i > 0 && copy == cudaSuccess) {
+                                                      Stage &s = ctx->stage[(i - 1) & 1];
+                                                      copy = cudaEventSynchronize(s.ev[0]);
+                                                      if (copy == cudaSuccess) bounceCopy(dst + (i - 1) * kPiece, s.hOut, len(i - 1));
+                                                    }
+                                                  }
+                                                  return copy == cudaSuccess;
+                                                },
+                                                out);
+  if (copy != cudaSuccess) return cudaFail(copy, "compressed bytes to the host");
+  if (!ok) return fail(SPZB200_ERR_INVALID, "%zu bytes do not fit the gzip block table", size);
+  return SPZB200_OK;
+}
+
+// No exception may cross the extern "C" boundary: allocation failures become SPZB200_ERR_NOMEM.
+template <class Fn>
+int guarded(const char *who, uint8_t **out, size_t *outSize, Fn &&fn) {
+  try {
+    return fn();
+  } catch (const std::exception &e) {
+    if (out) *out = nullptr;
+    if (outSize) *outSize = 0;
+    return fail(SPZB200_ERR_NOMEM, "%s: %s", who, e.what());
+  }
+}
+
+}  // namespace
+
+extern "C" {
+
+int spzb200_gzip_device(SpzB200Context *ctx, const uint8_t *data, size_t size, uint8_t **out, size_t *out_size, void *stream) {
+  const char *who = "spzb200_gzip_device";
+  if (!ctx) return fail(SPZB200_ERR_INVALID, "%s: null context", who);
+  if (!out || !out_size) return fail(SPZB200_ERR_INVALID, "%s: null output arguments", who);
+  *out = nullptr;
+  *out_size = 0;
+  if (!data && size) return fail(SPZB200_ERR_INVALID, "%s: null data", who);
+  return guarded(who, out, out_size, [&]() -> int {
+    CU(cudaSetDevice(ctx->device));
+    DeviceScratch scratch((cudaStream_t)stream);
+    uint8_t *slots = nullptr, *body = nullptr;
+    CU(scratch.alloc(&slots, spzb200::dfl::segmentCount(size) * spzb200::deflateSlotBytes()));
+    CU(scratch.alloc(&body, deflateBodyBytes(size)));
+    std::vector<uint8_t> bytes;
+    const int rc = gzipDeviceBytes(ctx, data, size, slots, body, scratch, &bytes);
+    return rc ? rc : handOverBytes(true, who, bytes, out, out_size);
+  });
+}
+
+int spzb200_save_spz_device(SpzB200Context *ctx, const SpzB200Cloud *in, int32_t from, int32_t antialiased, uint8_t **out,
+                            size_t *out_size, void *stream) {
+  const char *who = "spzb200_save_spz_device";
+  if (!ctx) return fail(SPZB200_ERR_INVALID, "%s: null context", who);
+  if (!out || !out_size) return fail(SPZB200_ERR_INVALID, "%s: null output arguments", who);
+  *out = nullptr;
+  *out_size = 0;
+  int rc = checkCloud(in, who);
+  if (rc) return rc;
+  if (in->num_points > std::numeric_limits<int32_t>::max())
+    return fail(SPZB200_ERR_INVALID, "%s: %lld points do not fit the container's 32-bit count", who, (long long)in->num_points);
+  if (from < 0 || from > 8) return fail(SPZB200_ERR_INVALID, "%s: coordinate system %d", who, from);
+  return guarded(who, out, out_size, [&]() -> int {
+    CU(cudaSetDevice(ctx->device));
+    const cudaStream_t st = (cudaStream_t)stream;
+    const size_t n = (size_t)in->num_points;
+    const int shDim = shDimOf(in->sh_degree);
+    size_t plane[6];  // struct order: positions, scales, rotations, alphas, colors, sh
+    bytePlaneBytes(shDim, SPZB200_STREAM_V3, plane);
+    for (size_t &b : plane) b *= n;
+    // container (stream order: positions, alphas, colors, scales, rotations, sh) after the 16 header bytes
+    const int streamOrder[6] = {0, 3, 4, 1, 2, 5};
+    size_t offset[6], total = spz::detail::kContainerHeaderBytes, aligned = 0;
+    for (int i = 0; i < 6; i++) {
+      offset[streamOrder[i]] = total;
+      total += plane[streamOrder[i]];
+      aligned += alignUp(plane[i], 16);
+    }
+    // Peak scratch: the slots (which first hold the encoder's aligned planes) + the container (which then holds the body).
+    const size_t segs = spzb200::dfl::segmentCount(total);
+    DeviceScratch scratch(st);
+    uint8_t *slots = nullptr, *container = nullptr;
+    CU(scratch.alloc(&slots, std::max(segs * spzb200::deflateSlotBytes(), aligned)));
+    CU(scratch.alloc(&container, deflateBodyBytes(total)));
+    SpzB200Packed packed;
+    std::memset(&packed, 0, sizeof packed);
+    packed.num_points = in->num_points;
+    packed.sh_degree = in->sh_degree;
+    uint8_t *planes[6], *p = slots;
+    for (int i = 0; i < 6; i++) {
+      planes[i] = p;
+      p += alignUp(plane[i], 16);
+    }
+    packed.positions = planes[0]; packed.scales = planes[1]; packed.rotations = planes[2];
+    packed.alphas = planes[3]; packed.colors = planes[4]; packed.sh = shDim ? planes[5] : nullptr;
+    if (n) {
+      const int erc = spzb200_encode_device_as(ctx, in, from, SPZB200_STREAM_V3, &packed, stream);
+      if (erc) return erc;
+    }
+    uint8_t header[spz::detail::kContainerHeaderBytes];
+    spz::detail::writeContainerHeader(3, in->num_points, in->sh_degree, antialiased != 0, header);
+    CU(spzb200::launchStoreBytes16(container, header, st));
+    ctx->kernelLaunches += 1;
+    for (int i = 0; i < 6; i++)
+      if (plane[i]) CU(cudaMemcpyAsync(container + offset[i], planes[i], plane[i], cudaMemcpyDeviceToDevice, st));
+    std::vector<uint8_t> bytes;
+    const int grc = gzipDeviceBytes(ctx, container, total, slots, container, scratch, &bytes);
+    return grc ? grc : handOverBytes(true, who, bytes, out, out_size);
+  });
+}
+
+int spzb200_spz_info(const uint8_t *bytes, size_t size, int64_t *num_points, int32_t *sh_degree) {
+  const char *who = "spzb200_spz_info";
+  if (!bytes || !num_points || !sh_degree) return fail(SPZB200_ERR_INVALID, "%s: null argument", who);
+  try {
+    std::vector<uint8_t> head;
+    if (!spz::detail::inflatePrefix(bytes, size, spz::detail::kContainerHeaderBytes, &head) ||
+        head.size() < spz::detail::kContainerHeaderBytes)
+      return fail(SPZB200_ERR_INVALID, "%s: not a gzip member holding an .spz header", who);
+    uint32_t words[3];
+    std::memcpy(words, head.data(), 12);
+    if (words[0] != spz::detail::kContainerMagic) return fail(SPZB200_ERR_INVALID, "%s: bad magic 0x%08x", who, words[0]);
+    if (words[1] < 1 || words[1] > 3) return fail(SPZB200_ERR_INVALID, "%s: container version %u not in 1..3", who, words[1]);
+    if (head[12] > 3) return fail(SPZB200_ERR_INVALID, "%s: SH degree %d not in 0..3", who, (int)head[12]);
+    *num_points = words[2];
+    *sh_degree = head[12];
+    return SPZB200_OK;
+  } catch (const std::exception &e) {
+    return fail(SPZB200_ERR_NOMEM, "%s: %s", who, e.what());
+  }
+}
+
+int spzb200_load_spz_device(SpzB200Context *ctx, const uint8_t *bytes, size_t size, int32_t to, SpzB200Cloud *out,
+                            int32_t *antialiased, void *stream) {
+  const char *who = "spzb200_load_spz_device";
+  if (!ctx) return fail(SPZB200_ERR_INVALID, "%s: null context", who);
+  if (!bytes || !out) return fail(SPZB200_ERR_INVALID, "%s: null argument", who);
+  if (to < 0 || to > 8) return fail(SPZB200_ERR_INVALID, "%s: coordinate system %d", who, to);
+  return guarded(who, nullptr, nullptr, [&]() -> int {
+    std::vector<uint8_t> container;
+    if (!spz::decompressGzippedParallel(bytes, size, spz::detail::inflateThreads(), &container))
+      return fail(SPZB200_ERR_INVALID, "%s: not a readable gzip member", who);
+    spz::detail::Container c;
+    if (!spz::detail::parseContainer(container.data(), container.size(), &c))
+      return fail(SPZB200_ERR_INVALID, "%s: not an .spz container (bad magic, version, degree or size)", who);
+    if (out->num_points != c.numPoints || out->sh_degree != c.shDegree)
+      return fail(SPZB200_ERR_INVALID, "%s: out holds %lld points of SH degree %d, the file %d of degree %d (spzb200_spz_info)", who,
+                  (long long)out->num_points, out->sh_degree, c.numPoints, c.shDegree);
+    int rc = checkCloud(out, who);
+    if (rc) return rc;
+    if (antialiased) *antialiased = c.antialiased ? 1 : 0;
+    if (c.numPoints == 0) return SPZB200_OK;
+    CU(cudaSetDevice(ctx->device));
+    const cudaStream_t st = (cudaStream_t)stream;
+    // stream order -> struct order (positions, scales, rotations, alphas, colors, sh)
+    const int structOf[6] = {0, 3, 4, 1, 2, 5};
+    size_t aligned = 0;
+    for (int i = 0; i < 6; i++) aligned += alignUp(c.bytes[i], 16);
+    DeviceScratch scratch(st);
+    uint8_t *base = nullptr;
+    CU(scratch.alloc(&base, aligned));
+    uint8_t *planes[6];
+    for (int i = 0; i < 6; i++) {
+      planes[structOf[i]] = base;
+      if (c.bytes[i]) CU(cudaMemcpyAsync(base, container.data() + c.offset[i], c.bytes[i], cudaMemcpyHostToDevice, st));
+      base += alignUp(c.bytes[i], 16);
+    }
+    SpzB200Packed in;
+    std::memset(&in, 0, sizeof in);
+    in.num_points = c.numPoints;
+    in.sh_degree = c.shDegree;
+    in.fractional_bits = c.fractionalBits;
+    in.version = c.half ? SPZB200_STREAM_V1 : c.smallestThree ? SPZB200_STREAM_V3 : SPZB200_STREAM_V2;
+    in.positions = planes[0]; in.scales = planes[1]; in.rotations = planes[2];
+    in.alphas = planes[3]; in.colors = planes[4]; in.sh = c.shDegree ? planes[5] : nullptr;
+    rc = spzb200_decode_device(ctx, &in, to, out, stream);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(st));
+    return SPZB200_OK;
+  });
 }
 
 }  // extern "C"

@@ -133,4 +133,14 @@ cudaError_t divisionSelfCheck(int part, unsigned long long pairsPerThread, unsig
 // saturates bytes the way the kernels assume (decided once per context).  `scratch` = one device int.
 cudaError_t probePackCvt(cudaStream_t stream, int *scratch, int *ok);
 
+// Device deflater (deflate_kernels.cu, DESIGN.md section 10): `size` device bytes at src ->
+// dfl::segmentCount(size) coded segments in slots (deflateSlotBytes() each), their byte counts and
+// CRC-32s, offsets[0..segments] (offsets[segments] = body bytes) and the packed raw deflate body
+// (at most size + 16 bytes per segment).  Three launches, asynchronous on `stream`.
+size_t deflateSlotBytes();
+cudaError_t launchDeflate(const uint8_t *src, unsigned long long size, uint8_t *slots, uint32_t *segBytes, uint32_t *segCrc,
+                          unsigned long long *offsets, uint8_t *body, cudaStream_t stream, int *launches);
+// 16 bytes from the host argument list to device memory, stream-ordered (no pageable copy, no sync).
+cudaError_t launchStoreBytes16(uint8_t *dst, const uint8_t bytes[16], cudaStream_t stream);
+
 }  // namespace spzb200

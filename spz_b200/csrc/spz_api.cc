@@ -81,9 +81,9 @@ using detail::resizeUninitialized;
 
 int shDimOf(int degree) { return degree == 0 ? 0 : degree == 1 ? 3 : degree == 2 ? 8 : degree == 3 ? 15 : 0; }
 
-constexpr uint32_t kMagic = 0x5053474e;  // "NGSP"
+constexpr uint32_t kMagic = detail::kContainerMagic;
 constexpr uint8_t kFlagAntialiased = 0x1;
-constexpr size_t kHeaderBytes = 16;
+constexpr size_t kHeaderBytes = detail::kContainerHeaderBytes;
 
 // ---- devices and contexts -----------------------------------------------------------------------
 // SPZ_B200_DEVICES="0,1,2,3" shards every call by point range over those GPUs (no collective);
@@ -244,10 +244,15 @@ int deflateThreads(size_t containerBytes) {
   if (env) return env;
   return containerBytes >= kAutoParallelGzipBytes ? hostThreads() : 1;
 }
+}  // namespace
+namespace detail {
 int inflateThreads() {
   const int env = gzipThreadsEnv();
   return env ? env : hostThreads();
 }
+}  // namespace detail
+namespace {
+using detail::inflateThreads;
 
 int64_t maxPointsToRead() {
   // The reference refuses more than 10,000,000 points (load-spz.cc:549).  Lifted here so the large
@@ -256,14 +261,9 @@ int64_t maxPointsToRead() {
   return std::numeric_limits<int32_t>::max();
 }
 
-// What the 16 header bytes and the stream length say (load-spz.cc:548-574), validated before anything is allocated.
-struct Container {
-  int32_t numPoints = 0, shDegree = 0, fractionalBits = 0;
-  bool antialiased = false, half = false, smallestThree = true;
-  size_t offset[6] = {0, 0, 0, 0, 0, 0};  // stream order: positions, alphas, colors, scales, rotations, sh
-  size_t bytes[6] = {0, 0, 0, 0, 0, 0};
-};
+}  // namespace
 
+namespace detail {
 bool parseContainer(const uint8_t *data, size_t size, Container *c) {
   if (size < kHeaderBytes) {
     logLine("[SPZ ERROR] deserializePackedGaussians: header not found");
@@ -310,6 +310,20 @@ bool parseContainer(const uint8_t *data, size_t size, Container *c) {
   c->antialiased = (flags & kFlagAntialiased) != 0;
   return true;
 }
+
+void writeContainerHeader(uint32_t version, int64_t numPoints, int32_t shDegree, bool antialiased, uint8_t out[kContainerHeaderBytes]) {
+  const uint32_t words[3] = {kContainerMagic, version, (uint32_t)numPoints};
+  std::memcpy(out, words, 12);
+  out[12] = (uint8_t)shDegree;
+  out[13] = 12;  // fractionalBits, load-spz.cc:270
+  out[14] = antialiased ? kFlagAntialiased : 0;
+  out[15] = 0;
+}
+}  // namespace detail
+
+namespace {
+using detail::Container;
+using detail::parseContainer;
 
 PackedGaussians deserialize(const uint8_t *data, size_t size) {
   Container c;
@@ -452,12 +466,7 @@ bool encodeContainer(const GaussianCloud &g, const PackOptions &o, int32_t strea
   stream->clear();
   resizeUninitialized(*stream, total);  // header written below, every plane byte by the encoder
   uint8_t *base = stream->data();
-  const uint32_t words[3] = {kMagic, s3 ? 3u : 2u, (uint32_t)g.numPoints};
-  std::memcpy(base, words, 12);
-  base[12] = (uint8_t)g.shDegree;
-  base[13] = 12;  // fractionalBits, load-spz.cc:270
-  base[14] = g.antialiased ? kFlagAntialiased : 0;
-  base[15] = 0;
+  detail::writeContainerHeader(s3 ? 3u : 2u, g.numPoints, g.shDegree, g.antialiased, base);
   *status = PackStatus::Ok;
   if (n == 0) return true;
   SpzB200Packed out;
@@ -768,6 +777,25 @@ bool decompressGzipped(const uint8_t *data, size_t size, std::vector<uint8_t> *o
   out->resize(produced);
   return true;
 }
+
+namespace detail {
+bool inflatePrefix(const uint8_t *data, size_t size, size_t want, std::vector<uint8_t> *out) {
+  out->assign(want, 0);
+  z_stream zs;
+  std::memset(&zs, 0, sizeof zs);
+  if (inflateInit2(&zs, 16 | MAX_WBITS) != Z_OK) return false;
+  zs.next_in = const_cast<Bytef *>(data);
+  zs.avail_in = (uInt)std::min<size_t>(size, (size_t)1 << 30);
+  zs.next_out = out->data();
+  zs.avail_out = (uInt)want;
+  int rc = Z_OK;
+  while (zs.avail_out > 0 && rc == Z_OK) rc = inflate(&zs, Z_NO_FLUSH);
+  const bool ok = zs.avail_out == 0 || rc == Z_STREAM_END;
+  out->resize(want - zs.avail_out);
+  inflateEnd(&zs);
+  return ok;
+}
+}  // namespace detail
 
 // zlib deflate with the reference's parameters (default level, gzip wrapper, memLevel 9,
 // load-spz.cc:186-214), so the compressed bytes are the same for the same input.

@@ -22,6 +22,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <exception>
+#include <functional>
 #include <thread>
 #include <vector>
 
@@ -151,32 +152,56 @@ bool compressGzippedParallel(const uint8_t *data, size_t size, int threads, std:
     return false;
   }
   uLong crc = crc32(0L, Z_NULL, 0);
-  size_t body = 0;
+  std::vector<uint32_t> compressed(blocks);
   for (size_t i = 0; i < blocks; i++) {
     crc = crc32_combine(crc, crcs[i], (z_off_t)std::min(blockSize, size - i * blockSize));
-    body += parts[i].size();
+    compressed[i] = (uint32_t)parts[i].size();
   }
-  const size_t subLen = 16 + 4 * blocks, xlen = 4 + subLen;
+  return detail::frameBlockMember(size, blockSize, compressed, (uint32_t)crc,
+                                  [&](uint8_t *dst) {
+                                    for (const auto &p : parts) {
+                                      if (!p.empty()) std::memcpy(dst, p.data(), p.size());
+                                      dst += p.size();
+                                    }
+                                    return true;
+                                  },
+                                  out);
+}
+
+namespace detail {
+bool frameBlockMember(size_t size, size_t blockSize, const std::vector<uint32_t> &compressed, uint32_t crc,
+                      const std::function<bool(uint8_t *)> &writeBody, std::vector<uint8_t> *out) {
+  const size_t blocks = compressed.size();
   out->clear();
-  out->reserve(12 + xlen + body + 8);
-  const uint8_t head[10] = {0x1f, 0x8b, 8, 4 /* FEXTRA */, 0, 0, 0, 0 /* mtime */, 0 /* xfl */, 3 /* unix */};
-  out->insert(out->end(), head, head + 10);
-  out->push_back((uint8_t)(xlen & 0xff));
-  out->push_back((uint8_t)(xlen >> 8));
-  out->push_back(kSubfieldId1);
-  out->push_back(kSubfieldId2);
-  out->push_back((uint8_t)(subLen & 0xff));
-  out->push_back((uint8_t)(subLen >> 8));
-  put32(out, (uint32_t)blockSize);
-  put32(out, (uint32_t)blocks);
-  put32(out, (uint32_t)(size & 0xffffffffu));
-  put32(out, (uint32_t)((uint64_t)size >> 32));
-  for (size_t i = 0; i < blocks; i++) put32(out, (uint32_t)parts[i].size());
-  for (size_t i = 0; i < blocks; i++) out->insert(out->end(), parts[i].begin(), parts[i].end());
-  put32(out, (uint32_t)crc);
-  put32(out, (uint32_t)(size & 0xffffffffu));
+  if (blocks == 0 || blocks > kMaxBlocks || blockSize == 0 || blockSize >= ((size_t)1 << 31)) return false;
+  size_t body = 0;
+  for (uint32_t c : compressed) body += c;
+  const size_t subLen = 16 + 4 * blocks, xlen = 4 + subLen;
+  std::vector<uint8_t> head = {0x1f, 0x8b, 8, 4 /* FEXTRA */, 0, 0, 0, 0 /* mtime */, 0 /* xfl */, 3 /* unix */};
+  head.push_back((uint8_t)(xlen & 0xff));
+  head.push_back((uint8_t)(xlen >> 8));
+  head.push_back(kSubfieldId1);
+  head.push_back(kSubfieldId2);
+  head.push_back((uint8_t)(subLen & 0xff));
+  head.push_back((uint8_t)(subLen >> 8));
+  put32(&head, (uint32_t)blockSize);
+  put32(&head, (uint32_t)blocks);
+  put32(&head, (uint32_t)(size & 0xffffffffu));
+  put32(&head, (uint32_t)((uint64_t)size >> 32));
+  for (size_t i = 0; i < blocks; i++) put32(&head, compressed[i]);
+  std::vector<uint8_t> tail;
+  put32(&tail, crc);
+  put32(&tail, (uint32_t)(size & 0xffffffffu));
+  resizeUninitialized(*out, head.size() + body + tail.size());  // the body is written in place, no zero-fill first
+  std::memcpy(out->data(), head.data(), head.size());
+  std::memcpy(out->data() + head.size() + body, tail.data(), tail.size());
+  if (body && !writeBody(out->data() + head.size())) {
+    out->clear();
+    return false;
+  }
   return true;
 }
+}  // namespace detail
 
 bool decompressGzippedParallel(const uint8_t *data, size_t size, int threads, std::vector<uint8_t> *out) {
   BlockTable t;

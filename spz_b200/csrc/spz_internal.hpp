@@ -2,6 +2,7 @@
 #pragma once
 #include <cstdint>
 #include <cstring>
+#include <functional>
 #include <string>
 #include <type_traits>
 #include <vector>
@@ -102,6 +103,35 @@ class ContextLease {
 std::vector<int32_t> configuredDevices();             // SPZ_B200_DEVICE(S)
 bool finishSpz(const PackedGaussians &packed, std::vector<uint8_t> *out);  // container + gzip (serial or SPZ_B200_GZIP_THREADS)
 void logLine(const char *fmt, ...);
+
+// Frames one gzip member in the block-table layout that compressGzippedParallel writes and
+// decompressGzippedParallel reads (spz_gzip.cc): header, FEXTRA "SZ" subfield {blockSize, block count,
+// 64-bit input size, compressed bytes of every block}, the concatenated raw deflate body -- written by
+// writeBody into the sum of `compressed` bytes at the pointer it is given -- then CRC-32 and ISIZE.  Every
+// block but the last inflates to blockSize bytes and ends byte-aligned.  Both writers (host zlib
+// threads, device deflater) call this.  false: at most 16000 blocks of less than 2 GiB, or writeBody failed.
+bool frameBlockMember(size_t size, size_t blockSize, const std::vector<uint32_t> &compressed, uint32_t crc,
+                      const std::function<bool(uint8_t *)> &writeBody, std::vector<uint8_t> *out);
+
+// What the 16 header bytes and the stream length of an inflated container say (load-spz.cc:548-574),
+// validated before anything is allocated: parseContainer logs and returns false the way the reference
+// fails.  offset / bytes are in stream order: positions, alphas, colors, scales, rotations, sh.
+struct Container {
+  int32_t numPoints = 0, shDegree = 0, fractionalBits = 0;
+  bool antialiased = false, half = false, smallestThree = true;
+  size_t offset[6] = {0, 0, 0, 0, 0, 0};
+  size_t bytes[6] = {0, 0, 0, 0, 0, 0};
+};
+bool parseContainer(const uint8_t *data, size_t size, Container *c);
+// Threads of the block-parallel inflater: SPZ_B200_GZIP_THREADS, else up to 16.
+int inflateThreads();
+// The first `want` bytes of the member's inflated stream (fewer if it is shorter); false if the gzip
+// data is not readable up to there.
+bool inflatePrefix(const uint8_t *data, size_t size, size_t want, std::vector<uint8_t> *out);
+constexpr size_t kContainerHeaderBytes = 16;
+constexpr uint32_t kContainerMagic = 0x5053474e;  // "NGSP"
+// The 16 header bytes the writer puts in front of the planes (load-spz.cc:131-139).
+void writeContainerHeader(uint32_t version, int64_t numPoints, int32_t shDegree, bool antialiased, uint8_t out[kContainerHeaderBytes]);
 
 }  // namespace detail
 }  // namespace spz
