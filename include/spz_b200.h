@@ -279,13 +279,35 @@ int spzb200_save_spz_device(SpzB200Context *ctx, const SpzB200Cloud *in /* devic
  * bytes), to size the output of spzb200_load_spz_device. */
 int spzb200_spz_info(const uint8_t *bytes, size_t size, int64_t *num_points, int32_t *sh_degree);
 
-/* loadSpz into caller-allocated DEVICE planes: inflates on the host (block-parallel for members with the
- * block table, serially for others such as the reference's files), validates the header the way loadSpz
- * does before anything is allocated, copies each plane to the device and decodes it with the device
- * decoder (container versions 1-3).  out->num_points and out->sh_degree must be what spzb200_spz_info
- * reports.  `to` is UnpackOptions::to; *antialiased (may be NULL) receives the header flag.  A file that
- * does not inflate or parse fails with SPZB200_ERR_INVALID and leaves `out` untouched.  Device scratch:
- * the packed planes (the container's size).  Returns when `out` is complete. */
+/* Inflated size and block count of a gzip member carrying the "SZ" block table (what spzb200_gzip with
+ * threads > 1, saveSpz from 8 MiB, spzb200_gzip_device and spzb200_save_spz_device write).  No GPU.
+ * SPZB200_ERR_INVALID for a member without the table or with one the parallel inflater would not trust. */
+int spzb200_gzip_table_info(const uint8_t *bytes, size_t size, uint64_t *inflated_size, int64_t *blocks);
+
+/* The inflate stage on the device: a block-table gzip member in HOST memory -> its inflated bytes at
+ * `out` (DEVICE, out_capacity >= the table's size).  The compressed bytes cross PCIe; each table block
+ * is inflated by the device and the CRC-32 and ISIZE are checked.  The result is exactly what
+ * spzb200_gunzip(threads > 1) returns for the same bytes, and the call fails where that fails: when the device cannot
+ * vouch for a block, the host inflater produces the bytes.  *on_device (may be NULL) = 1 when the device
+ * produced them.  Synchronous, after earlier work on `stream`.  A member without the table fails with
+ * SPZB200_ERR_INVALID before anything is allocated; after a failure the contents of `out` are undefined.
+ * Device scratch: the compressed body. */
+int spzb200_gunzip_device(SpzB200Context *ctx, const uint8_t *bytes, size_t size, uint8_t *out,
+                          size_t out_capacity, size_t *out_size, int32_t *on_device, void *stream);
+
+/* loadSpz into caller-allocated DEVICE planes (container versions 1-3).  out->num_points and
+ * out->sh_degree must be what spzb200_spz_info reports.  `to` is UnpackOptions::to; *antialiased (may be
+ * NULL) receives the header flag.  A member whose block table has blocks of less than 1 MiB (every
+ * spzb200_save_spz_device file) is inflated on the device: its header is validated the way loadSpz does
+ * before anything is allocated, only the compressed bytes cross PCIe, and the planes are moved into
+ * aligned places on the device and decoded there.  Other members (the reference's files, saveSpz files,
+ * whose zlib blocks of 1 MiB or more the host inflates faster), and any member the device cannot vouch
+ * for, take the host route: inflate on the host (block-parallel where a table allows), validate, copy
+ * each plane up and decode on the device.
+ * Both routes give the same verdict and the same planes.  A file that does not inflate or parse fails
+ * with SPZB200_ERR_INVALID and leaves `out` untouched.  Device scratch: the container and its packed
+ * planes (twice the container's size) plus the compressed body on the device route, the packed planes
+ * on the host route.  Returns when `out` is complete. */
 int spzb200_load_spz_device(SpzB200Context *ctx, const uint8_t *bytes /* host */, size_t size, int32_t to,
                             SpzB200Cloud *out /* device */, int32_t *antialiased, void *stream);
 

@@ -79,6 +79,9 @@ SIGNATURES = {
                                           C.c_void_p]),
     "spzb200_spz_info": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(C.c_int64), C.POINTER(C.c_int32)]),
     "spzb200_load_spz_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int32, C.POINTER(Cloud), C.POINTER(C.c_int32), C.c_void_p]),
+    "spzb200_gzip_table_info": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(C.c_uint64), C.POINTER(C.c_int64)]),
+    "spzb200_gunzip_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t),
+                                        C.POINTER(C.c_int32), C.c_void_p]),
     "spzb200_shard_range": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "spzb200_tile_gaussians": (C.c_int32, [C.c_int32]),
     "spzb200_flip_bits": (None, [C.c_int32, C.c_int32, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),

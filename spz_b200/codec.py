@@ -201,6 +201,15 @@ def spz_info(blob):
     return n.value, deg.value
 
 
+def gzip_table_info(blob):
+    """(inflated_size, blocks) of a gzip member carrying the "SZ" block table (spzb200_gzip_table_info; no
+    GPU).  CodecError(ERR_INVALID) for a member without one, or with one the parallel inflater would not trust."""
+    buf = np.frombuffer(blob, np.uint8) if not isinstance(blob, np.ndarray) else np.ascontiguousarray(blob, np.uint8)
+    size, blocks = C.c_uint64(0), C.c_int64(0)
+    N.check(N.lib().spzb200_gzip_table_info(C.c_void_p(buf.ctypes.data if buf.size else None), buf.size, C.byref(size), C.byref(blocks)))
+    return size.value, blocks.value
+
+
 def shard_range(n: int, sh_degree: int, num_shards: int, index: int):
     """Contiguous point range of one shard (host logic, no GPU): spzb200_shard_range."""
     a, b = C.c_int64(0), C.c_int64(0)
@@ -346,6 +355,22 @@ class Context:
         rc = N.lib().spzb200_gzip_device(self._h, C.c_void_p(ptr), data.numel(), C.byref(out), C.byref(size),
                                          C.c_void_p(self._stream_handle(stream)))
         return self._take_bytes(rc, out, size)
+
+    def gunzip_device(self, blob, out=None, stream=None):
+        """A block-table gzip member in host memory -> (uint8 CUDA tensor of its inflated bytes, on_device), via
+        spzb200_gunzip_device: the bytes spzb200_gunzip(threads > 1) returns; on_device is True when the device
+        inflater produced them.  `out`, if given, is a contiguous uint8 CUDA tensor of at least the inflated
+        size; the result is its leading slice.  Otherwise one is allocated from the table's size."""
+        buf = np.frombuffer(blob, np.uint8) if not isinstance(blob, np.ndarray) else np.ascontiguousarray(blob, np.uint8)
+        if out is None:
+            import torch
+            size, _ = gzip_table_info(buf)
+            out = torch.empty(size, dtype=torch.uint8, device=f"cuda:{self.device}")
+        ptr = _ptr(out, "u1", out.numel(), True, "out")
+        got, on_device = C.c_size_t(0), C.c_int32(0)
+        N.check(N.lib().spzb200_gunzip_device(self._h, C.c_void_p(buf.ctypes.data if buf.size else None), buf.size, C.c_void_p(ptr),
+                                              out.numel(), C.byref(got), C.byref(on_device), C.c_void_p(self._stream_handle(stream))))
+        return out[:got.value], bool(on_device.value)
 
     def save_spz_device(self, cloud: CloudPlanes, frm: int = 0, antialiased: bool = False, stream=None) -> bytes:
         """The .spz file of a device cloud (spzb200_save_spz_device): what saveSpz writes, inflated."""

@@ -35,6 +35,7 @@
 #include "codec_kernels.cuh"
 #include "codec_math.cuh"
 #include "deflate_format.cuh"
+#include "inflate_format.cuh"
 #include "spz_internal.hpp"
 
 namespace {
@@ -1927,6 +1928,48 @@ struct DeviceScratch {
 
 size_t deflateBodyBytes(size_t size) { return size + 16 * spzb200::dfl::segmentCount(size) + 16; }
 
+// `bytes` between pageable host memory and the device, stream-ordered after earlier work on `stream`, in
+// pieces through two of the context's pinned bounce buffers: the DMA of one piece overlaps the host copy
+// of the next (a pageable copy of a whole compressed body ran at ~2 GB/s on a B200 host).  Synchronous.
+int bouncedCopy(SpzB200Context *ctx, void *dst, const void *src, size_t bytes, cudaMemcpyKind kind, cudaStream_t stream) {
+  constexpr size_t kPiece = (size_t)8 << 20;
+  const bool down = kind == cudaMemcpyDeviceToHost;
+  for (int k = 0; k < 2; k++) {
+    Stage &s = ctx->stage[k];
+    const int rc = down ? ensureBounce(s.hOut, s.hOutCap, kPiece) : ensureBounce(s.hIn, s.hInCap, kPiece);
+    if (rc) return rc;
+  }
+  uint8_t *to = static_cast<uint8_t *>(dst);
+  const uint8_t *from = static_cast<const uint8_t *>(src);
+  const size_t pieces = (bytes + kPiece - 1) / kPiece;
+  auto len = [&](size_t i) { return std::min(kPiece, bytes - i * kPiece); };
+  if (down) {  // queue piece i, then copy piece i - 1 out of its buffer
+    for (size_t i = 0; i <= pieces; i++) {
+      if (i < pieces) {
+        Stage &s = ctx->stage[i & 1];
+        CU(cudaMemcpyAsync(s.hOut, from + i * kPiece, len(i), cudaMemcpyDeviceToHost, stream));
+        CU(cudaEventRecord(s.ev[0], stream));
+      }
+      if (i > 0) {
+        Stage &s = ctx->stage[(i - 1) & 1];
+        CU(cudaEventSynchronize(s.ev[0]));
+        bounceCopy(to + (i - 1) * kPiece, s.hOut, len(i - 1));
+      }
+    }
+    return SPZB200_OK;
+  }
+  // up: wait until the buffer's previous DMA is done, fill it, queue its DMA
+  for (size_t i = 0; i < pieces; i++) {
+    Stage &s = ctx->stage[i & 1];
+    if (i >= 2) CU(cudaEventSynchronize(s.ev[0]));
+    bounceCopy(s.hIn, from + i * kPiece, len(i));
+    CU(cudaMemcpyAsync(to + i * kPiece, s.hIn, len(i), cudaMemcpyHostToDevice, stream));
+    CU(cudaEventRecord(s.ev[0], stream));
+  }
+  CU(cudaStreamSynchronize(stream));
+  return SPZB200_OK;
+}
+
 // `size` device bytes at src -> one gzip member in *out.  slots: segmentCount * deflateSlotBytes() bytes; body:
 // deflateBodyBytes(size) bytes (may be src itself: the body is written after the last read of src).  Synchronous.
 int gzipDeviceBytes(SpzB200Context *ctx, const uint8_t *src, size_t size, uint8_t *slots, uint8_t *body, DeviceScratch &scratch,
@@ -1952,36 +1995,54 @@ int gzipDeviceBytes(SpzB200Context *ctx, const uint8_t *src, size_t size, uint8_
     crc = crc32_combine(crc, hostSeg[segs + s], (z_off_t)len);
     blockBytes[s / perBlock] += hostSeg[s];
   }
-  // The body comes back in pieces through two of the context's pinned bounce buffers: the DMA of one piece
-  // overlaps the host copy of the previous one (a pageable D2H of the whole body ran at ~2 GB/s on a B200 host).
-  constexpr size_t kPiece = (size_t)8 << 20;
-  int brc = SPZB200_OK;
-  for (int k = 0; k < 2 && brc == SPZB200_OK; k++) brc = ensureBounce(ctx->stage[k].hOut, ctx->stage[k].hOutCap, kPiece);
-  if (brc) return brc;
-  cudaError_t copy = cudaSuccess;
+  int copyRc = SPZB200_OK;
   const bool ok = spz::detail::frameBlockMember(size, perBlock * dfl::kSegBytes, blockBytes, (uint32_t)crc,
                                                 [&](uint8_t *dst) {
                                                   size_t total = 0;
                                                   for (uint32_t b : blockBytes) total += b;
-                                                  const size_t pieces = (total + kPiece - 1) / kPiece;
-                                                  auto len = [&](size_t i) { return std::min(kPiece, total - i * kPiece); };
-                                                  for (size_t i = 0; i <= pieces && copy == cudaSuccess; i++) {
-                                                    if (i < pieces) {
-                                                      Stage &s = ctx->stage[i & 1];
-                                                      copy = cudaMemcpyAsync(s.hOut, body + i * kPiece, len(i), cudaMemcpyDeviceToHost, scratch.stream);
-                                                      if (copy == cudaSuccess) copy = cudaEventRecord(s.ev[0], scratch.stream);
-                                                    }
-                                                    if (i > 0 && copy == cudaSuccess) {
-                                                      Stage &s = ctx->stage[(i - 1) & 1];
-                                                      copy = cudaEventSynchronize(s.ev[0]);
-                                                      if (copy == cudaSuccess) bounceCopy(dst + (i - 1) * kPiece, s.hOut, len(i - 1));
-                                                    }
-                                                  }
-                                                  return copy == cudaSuccess;
+                                                  copyRc = bouncedCopy(ctx, dst, body, total, cudaMemcpyDeviceToHost, scratch.stream);
+                                                  return copyRc == SPZB200_OK;
                                                 },
                                                 out);
-  if (copy != cudaSuccess) return cudaFail(copy, "compressed bytes to the host");
+  if (copyRc) return copyRc;
   if (!ok) return fail(SPZB200_ERR_INVALID, "%zu bytes do not fit the gzip block table", size);
+  return SPZB200_OK;
+}
+
+// The inflate stage on the device: the table blocks of the member at `bytes` (parsed into t) -> dOut
+// (t.totalSize bytes).  The compressed body crosses PCIe through the bounce buffers, one kernel inflates
+// every block and checksums its slice, and the host combines the CRCs.  *vouched: every block filled
+// its slice exactly and the combined CRC-32 matches the trailer (ISIZE was checked by the parser); when
+// false, dOut holds nothing to use and the host inflater has to give the verdict.  Synchronous.
+int inflateDeviceBytes(SpzB200Context *ctx, const uint8_t *bytes, const spz::detail::BlockTable &t, uint8_t *dOut,
+                       DeviceScratch &scratch, bool *vouched) {
+  *vouched = false;
+  const size_t blocks = t.compressed.size();
+  std::vector<unsigned long long> offset(blocks + 1, 0);
+  for (size_t i = 0; i < blocks; i++) offset[i + 1] = offset[i] + t.compressed[i];
+  uint8_t *body = nullptr;
+  unsigned long long *dOffset = nullptr;
+  uint32_t *dCrc = nullptr;
+  CU(scratch.alloc(&body, offset[blocks]));
+  CU(scratch.alloc(&dOffset, (blocks + 1) * sizeof(unsigned long long)));
+  CU(scratch.alloc(&dCrc, 2 * blocks * sizeof(uint32_t)));
+  int32_t *dStatus = reinterpret_cast<int32_t *>(dCrc + blocks);
+  CU(cudaMemcpyAsync(dOffset, offset.data(), (blocks + 1) * sizeof(unsigned long long), cudaMemcpyHostToDevice, scratch.stream));
+  const int rc = bouncedCopy(ctx, body, bytes + t.bodyOffset, offset[blocks], cudaMemcpyHostToDevice, scratch.stream);
+  if (rc) return rc;
+  int warps = 0;
+  CU(spzb200::launchInflate(body, dOffset, (long long)blocks, t.blockSize, t.totalSize, dOut, dCrc, dStatus, ctx->smCount,
+                            scratch.stream, &warps));
+  ctx->kernelLaunches += 1;
+  std::vector<uint32_t> result(2 * blocks);
+  CU(cudaMemcpyAsync(result.data(), dCrc, 2 * blocks * sizeof(uint32_t), cudaMemcpyDeviceToHost, scratch.stream));
+  CU(cudaStreamSynchronize(scratch.stream));
+  uLong crc = crc32(0L, Z_NULL, 0);
+  for (size_t i = 0; i < blocks; i++) {
+    if (result[blocks + i] != spzb200::ifl::kOk) return SPZB200_OK;
+    crc = crc32_combine(crc, result[i], (z_off_t)t.blockBytes(i));
+  }
+  *vouched = (uint32_t)crc == t.crc;
   return SPZB200_OK;
 }
 
@@ -2102,6 +2163,126 @@ int spzb200_spz_info(const uint8_t *bytes, size_t size, int64_t *num_points, int
   }
 }
 
+int spzb200_gzip_table_info(const uint8_t *bytes, size_t size, uint64_t *inflated_size, int64_t *blocks) {
+  const char *who = "spzb200_gzip_table_info";
+  if (!bytes || !inflated_size || !blocks) return fail(SPZB200_ERR_INVALID, "%s: null argument", who);
+  try {
+    spz::detail::BlockTable t;
+    if (!spz::detail::parseBlockTable(bytes, size, &t))
+      return fail(SPZB200_ERR_INVALID, "%s: not a gzip member with a block table the parallel inflater trusts", who);
+    *inflated_size = t.totalSize;
+    *blocks = (int64_t)t.compressed.size();
+    return SPZB200_OK;
+  } catch (const std::exception &e) {
+    return fail(SPZB200_ERR_NOMEM, "%s: %s", who, e.what());
+  }
+}
+
+int spzb200_gunzip_device(SpzB200Context *ctx, const uint8_t *bytes, size_t size, uint8_t *out, size_t out_capacity, size_t *out_size,
+                          int32_t *on_device, void *stream) {
+  const char *who = "spzb200_gunzip_device";
+  if (!ctx) return fail(SPZB200_ERR_INVALID, "%s: null context", who);
+  if (!bytes || !out || !out_size) return fail(SPZB200_ERR_INVALID, "%s: null argument", who);
+  *out_size = 0;
+  if (on_device) *on_device = 0;
+  return guarded(who, nullptr, nullptr, [&]() -> int {
+    spz::detail::BlockTable t;
+    if (!spz::detail::parseBlockTable(bytes, size, &t))
+      return fail(SPZB200_ERR_INVALID, "%s: not a gzip member with a block table the parallel inflater trusts", who);
+    if (out_capacity < t.totalSize)
+      return fail(SPZB200_ERR_INVALID, "%s: out holds %zu bytes, the member inflates to %llu", who, out_capacity,
+                  (unsigned long long)t.totalSize);
+    CU(cudaSetDevice(ctx->device));
+    const cudaStream_t st = (cudaStream_t)stream;
+    bool vouched = false;
+    {
+      DeviceScratch scratch(st);
+      const int rc = inflateDeviceBytes(ctx, bytes, t, out, scratch, &vouched);
+      if (rc) return rc;
+    }
+    if (!vouched) {  // the host inflater's verdict and bytes; they must fill exactly what the table announced
+      std::vector<uint8_t> host;
+      if (!spz::decompressGzippedParallel(bytes, size, spz::detail::inflateThreads(), &host))
+        return fail(SPZB200_ERR_INVALID, "%s: not a readable gzip member", who);
+      if (host.size() != t.totalSize)
+        return fail(SPZB200_ERR_INVALID, "%s: the member inflates to %zu bytes, its block table says %llu", who, host.size(),
+                    (unsigned long long)t.totalSize);
+      const int rc = bouncedCopy(ctx, out, host.data(), host.size(), cudaMemcpyHostToDevice, st);
+      if (rc) return rc;
+    }
+    *out_size = (size_t)t.totalSize;
+    if (on_device) *on_device = vouched ? 1 : 0;
+    return SPZB200_OK;
+  });
+}
+
+}  // extern "C"
+
+namespace {
+
+// Table blocks from this size up are loaded through the host route.  Each block is one serial decode on
+// the device, so few large blocks leave most of the GPU idle: a 10M SH3 file of 620 zlib blocks of 1 MiB
+// (saveSpz) loads in 339 ms on the device route against 293 ms on the host route, while the 9919 blocks
+// of 64 KiB of a save_spz_device file load in 129 ms against 262 ms (B200 at 1000 W,
+// profiles/r4_device_inflate_timing_unrouted.jsonl; DESIGN.md section 10b).
+constexpr size_t kDeviceLoadMaxBlock = (size_t)1 << 20;
+
+// load_spz_device for a member with a block table: the container is inflated on the device, its planes
+// are moved to 16-byte-aligned places and decoded.  *taken = false (and `out` untouched) whenever this
+// route cannot finish the call -- the header or the table disagree with `out`, the device cannot vouch
+// for a block, an allocation fails -- and the caller then runs the host route, whose verdict is the
+// call's.  After *taken = true the result is the call's result.
+int loadSpzDeviceInflated(SpzB200Context *ctx, const uint8_t *bytes, size_t size, const spz::detail::BlockTable &t, int32_t to,
+                          SpzB200Cloud *out, int32_t *antialiased, void *stream, bool *taken) {
+  *taken = false;
+  std::vector<uint8_t> head;
+  if (!spz::detail::inflatePrefix(bytes, size, spz::detail::kContainerHeaderBytes, &head) || head.size() < spz::detail::kContainerHeaderBytes)
+    return SPZB200_OK;
+  spz::detail::Container c;
+  if (!spz::detail::parseContainer(head.data(), (size_t)t.totalSize, &c)) return SPZB200_OK;  // reads the 16 bytes and the size
+  if (out->num_points != c.numPoints || out->sh_degree != c.shDegree || c.numPoints == 0) return SPZB200_OK;
+  if (checkCloud(out, "spzb200_load_spz_device")) return SPZB200_OK;
+  if (cudaSetDevice(ctx->device) != cudaSuccess) return SPZB200_OK;
+  const cudaStream_t st = (cudaStream_t)stream;
+  // stream order -> struct order (positions, scales, rotations, alphas, colors, sh)
+  const int structOf[6] = {0, 3, 4, 1, 2, 5};
+  size_t aligned = 0;
+  for (int i = 0; i < 6; i++) aligned += alignUp(c.bytes[i], 16);
+  DeviceScratch scratch(st);
+  uint8_t *container = nullptr, *base = nullptr;
+  if (scratch.alloc(&container, (size_t)t.totalSize) != cudaSuccess || scratch.alloc(&base, aligned) != cudaSuccess) {
+    cudaGetLastError();
+    return SPZB200_OK;
+  }
+  bool vouched = false;
+  if (inflateDeviceBytes(ctx, bytes, t, container, scratch, &vouched) != SPZB200_OK || !vouched) return SPZB200_OK;
+  // From here on the call's result is this route's: the container is what the host route would inflate.
+  *taken = true;
+  if (antialiased) *antialiased = c.antialiased ? 1 : 0;
+  uint8_t *planes[6];
+  for (int i = 0; i < 6; i++) {  // plane offsets such as 16 + 9n are not aligned: move the planes
+    planes[structOf[i]] = base;
+    if (c.bytes[i]) CU(cudaMemcpyAsync(base, container + c.offset[i], c.bytes[i], cudaMemcpyDeviceToDevice, st));
+    base += alignUp(c.bytes[i], 16);
+  }
+  SpzB200Packed in;
+  std::memset(&in, 0, sizeof in);
+  in.num_points = c.numPoints;
+  in.sh_degree = c.shDegree;
+  in.fractional_bits = c.fractionalBits;
+  in.version = c.half ? SPZB200_STREAM_V1 : c.smallestThree ? SPZB200_STREAM_V3 : SPZB200_STREAM_V2;
+  in.positions = planes[0]; in.scales = planes[1]; in.rotations = planes[2];
+  in.alphas = planes[3]; in.colors = planes[4]; in.sh = c.shDegree ? planes[5] : nullptr;
+  const int rc = spzb200_decode_device(ctx, &in, to, out, stream);
+  if (rc) return rc;
+  CU(cudaStreamSynchronize(st));
+  return SPZB200_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
 int spzb200_load_spz_device(SpzB200Context *ctx, const uint8_t *bytes, size_t size, int32_t to, SpzB200Cloud *out,
                             int32_t *antialiased, void *stream) {
   const char *who = "spzb200_load_spz_device";
@@ -2109,6 +2290,17 @@ int spzb200_load_spz_device(SpzB200Context *ctx, const uint8_t *bytes, size_t si
   if (!bytes || !out) return fail(SPZB200_ERR_INVALID, "%s: null argument", who);
   if (to < 0 || to > 8) return fail(SPZB200_ERR_INVALID, "%s: coordinate system %d", who, to);
   return guarded(who, nullptr, nullptr, [&]() -> int {
+    {
+      spz::detail::BlockTable t;
+      if (spz::detail::parseBlockTable(bytes, size, &t) && t.blockSize < kDeviceLoadMaxBlock) {
+        bool taken = false;
+        const int rc = loadSpzDeviceInflated(ctx, bytes, size, t, to, out, antialiased, stream, &taken);
+        if (taken) return rc;
+      }
+    }
+    // Members without a block table (the reference's files, small saveSpz files), with blocks of 1 MiB or
+    // more (saveSpz's zlib blocks), and those the device route could not finish: inflate on the host, copy
+    // the container's planes up, decode on the device.
     std::vector<uint8_t> container;
     if (!spz::decompressGzippedParallel(bytes, size, spz::detail::inflateThreads(), &container))
       return fail(SPZB200_ERR_INVALID, "%s: not a readable gzip member", who);

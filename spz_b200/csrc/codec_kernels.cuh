@@ -143,4 +143,13 @@ cudaError_t launchDeflate(const uint8_t *src, unsigned long long size, uint8_t *
 // 16 bytes from the host argument list to device memory, stream-ordered (no pageable copy, no sync).
 cudaError_t launchStoreBytes16(uint8_t *dst, const uint8_t bytes[16], cudaStream_t stream);
 
+// Device inflater (inflate_kernels.cu, DESIGN.md section 10): table block i of a block-table gzip
+// member -- raw deflate bytes body[inOffset[i], inOffset[i + 1]) -- into out[i * blockSize, ...) (the
+// last block holds total - (blocks - 1) * blockSize bytes).  status[i] = ifl::kOk when the block filled
+// its slice exactly, crc[i] its CRC-32 then.  One launch, asynchronous on `stream`; *warpsPerCta is
+// the geometry chosen for the block count and SM count.
+cudaError_t launchInflate(const uint8_t *body, const unsigned long long *inOffset, long long blocks, unsigned long long blockSize,
+                          unsigned long long total, uint8_t *out, uint32_t *crc, int32_t *status, int smCount, cudaStream_t stream,
+                          int *warpsPerCta);
+
 }  // namespace spzb200

@@ -84,52 +84,6 @@ bool deflateBlock(const uint8_t *src, size_t len, bool last, int level, std::vec
   return ok;
 }
 
-struct BlockTable {
-  size_t blockSize = 0;
-  uint64_t totalSize = 0;            // uncompressed bytes of the whole member
-  std::vector<uint32_t> compressed;  // bytes of each block's deflate data
-  size_t bodyOffset = 0;             // where the deflate data starts
-};
-
-// Parses the gzip header; returns true and fills `t` when it carries our block table.
-bool findBlockTable(const uint8_t *d, size_t n, BlockTable *t) {
-  if (n < 18 || d[0] != 0x1f || d[1] != 0x8b || d[2] != 8) return false;
-  const uint8_t flg = d[3];
-  size_t pos = 10;
-  bool found = false;
-  if (flg & 4) {  // FEXTRA
-    if (pos + 2 > n) return false;
-    const size_t xlen = d[pos] | (d[pos + 1] << 8);
-    pos += 2;
-    if (pos + xlen > n) return false;
-    size_t p = pos;
-    while (p + 4 <= pos + xlen) {
-      const size_t len = d[p + 2] | (d[p + 3] << 8);
-      if (p + 4 + len > pos + xlen) break;
-      if (d[p] == kSubfieldId1 && d[p + 1] == kSubfieldId2 && len >= 16 && (len - 16) % 4 == 0) {
-        const uint8_t *q = d + p + 4;
-        t->blockSize = get32(q);
-        const size_t blocks = get32(q + 4);
-        t->totalSize = (uint64_t)get32(q + 8) | ((uint64_t)get32(q + 12) << 32);
-        if (blocks * 4 + 16 == len && t->blockSize > 0 && blocks > 0 &&
-            t->totalSize > (uint64_t)(blocks - 1) * t->blockSize && t->totalSize <= (uint64_t)blocks * t->blockSize) {
-          t->compressed.resize(blocks);
-          for (size_t i = 0; i < blocks; i++) t->compressed[i] = get32(q + 16 + 4 * i);
-          found = true;
-        }
-      }
-      p += 4 + len;
-    }
-    pos += xlen;
-  }
-  if (flg & 8) { while (pos < n && d[pos]) pos++; pos++; }   // FNAME
-  if (flg & 16) { while (pos < n && d[pos]) pos++; pos++; }  // FCOMMENT
-  if (flg & 2) pos += 2;                                     // FHCRC
-  if (pos > n) return false;
-  t->bodyOffset = pos;
-  return found;
-}
-
 }  // namespace
 
 bool compressGzippedParallel(const uint8_t *data, size_t size, int threads, std::vector<uint8_t> *out) {
@@ -201,28 +155,70 @@ bool frameBlockMember(size_t size, size_t blockSize, const std::vector<uint32_t>
   }
   return true;
 }
+
+// Parses the gzip header; true when it carries the block table and the table is one the block-parallel
+// inflaters may trust.  The table is untrusted input and sizes the output before a byte has been
+// inflated, so besides fitting the member (blocks, then CRC-32 and ISIZE) it must agree with ISIZE, keep
+// every block under 2 GiB (zlib counts a block in 32 bits) and claim no block larger than deflate can
+// expand its compressed length to: 1032 : 1 (a 258-byte match costs at least 2 bits).  Otherwise the
+// serial inflater, whose buffer only grows with what zlib really produces, gives the verdict.
+bool parseBlockTable(const uint8_t *d, size_t n, BlockTable *t) {
+  if (n < 18 || d[0] != 0x1f || d[1] != 0x8b || d[2] != 8) return false;
+  const uint8_t flg = d[3];
+  size_t pos = 10;
+  bool found = false;
+  if (flg & 4) {  // FEXTRA
+    if (pos + 2 > n) return false;
+    const size_t xlen = d[pos] | (d[pos + 1] << 8);
+    pos += 2;
+    if (pos + xlen > n) return false;
+    size_t p = pos;
+    while (p + 4 <= pos + xlen) {
+      const size_t len = d[p + 2] | (d[p + 3] << 8);
+      if (p + 4 + len > pos + xlen) break;
+      if (d[p] == kSubfieldId1 && d[p + 1] == kSubfieldId2 && len >= 16 && (len - 16) % 4 == 0) {
+        const uint8_t *q = d + p + 4;
+        t->blockSize = get32(q);
+        const size_t blocks = get32(q + 4);
+        t->totalSize = (uint64_t)get32(q + 8) | ((uint64_t)get32(q + 12) << 32);
+        if (blocks * 4 + 16 == len && t->blockSize > 0 && blocks > 0 &&
+            t->totalSize > (uint64_t)(blocks - 1) * t->blockSize && t->totalSize <= (uint64_t)blocks * t->blockSize) {
+          t->compressed.resize(blocks);
+          for (size_t i = 0; i < blocks; i++) t->compressed[i] = get32(q + 16 + 4 * i);
+          found = true;
+        }
+      }
+      p += 4 + len;
+    }
+    pos += xlen;
+  }
+  if (flg & 8) { while (pos < n && d[pos]) pos++; pos++; }   // FNAME
+  if (flg & 16) { while (pos < n && d[pos]) pos++; pos++; }  // FCOMMENT
+  if (flg & 2) pos += 2;                                     // FHCRC
+  if (pos > n || !found || t->compressed.empty()) return false;
+  t->bodyOffset = pos;
+  const size_t blocks = t->compressed.size();
+  size_t end = pos;
+  for (size_t i = 0; i < blocks; i++) end += t->compressed[i];
+  if (end + 8 > n) return false;  // the table does not fit: not ours after all
+  t->crc = get32(d + end);
+  if ((uint32_t)(t->totalSize & 0xffffffffu) != get32(d + end + 4)) return false;
+  constexpr uint64_t kMaxExpansion = 1032;
+  if (t->blockSize >= ((size_t)1 << 31)) return false;
+  for (size_t i = 0; i < blocks; i++)
+    if (t->blockBytes(i) > kMaxExpansion * ((uint64_t)t->compressed[i] + 1)) return false;
+  return true;
+}
 }  // namespace detail
 
 bool decompressGzippedParallel(const uint8_t *data, size_t size, int threads, std::vector<uint8_t> *out) {
-  BlockTable t;
-  if (threads <= 1 || !findBlockTable(data, size, &t) || t.compressed.empty()) return decompressGzipped(data, size, out);
+  detail::BlockTable t;
+  if (threads <= 1 || !detail::parseBlockTable(data, size, &t)) return decompressGzipped(data, size, out);
   const size_t blocks = t.compressed.size();
   std::vector<size_t> offset(blocks + 1, t.bodyOffset);
   for (size_t i = 0; i < blocks; i++) offset[i + 1] = offset[i] + t.compressed[i];
-  if (offset[blocks] + 8 > size) return decompressGzipped(data, size, out);  // table does not fit: not ours after all
-  const uint32_t wantCrc = get32(data + offset[blocks]), isize = get32(data + offset[blocks] + 4);
-  const size_t total = (size_t)t.totalSize, lastLen = total - (blocks - 1) * t.blockSize;
-  if ((uint32_t)(total & 0xffffffffu) != isize) return decompressGzipped(data, size, out);
-  // The table is untrusted input and sizes the allocation below before a byte has been inflated.
-  // Deflate cannot expand by more than 1032 : 1 (a 258-byte match costs at least 2 bits), so a block
-  // that claims more than that for its compressed length -- and with it any absurd total -- is not
-  // ours: the serial inflater, whose buffer only grows with what zlib really produces, gives the verdict.
-  constexpr uint64_t kMaxExpansion = 1032;
-  if (t.blockSize >= ((size_t)1 << 31)) return decompressGzipped(data, size, out);  // zlib counts a block in 32 bits
-  for (size_t i = 0; i < blocks; i++) {
-    const uint64_t len = i + 1 == blocks ? lastLen : t.blockSize;
-    if (len > kMaxExpansion * ((uint64_t)t.compressed[i] + 1)) return decompressGzipped(data, size, out);
-  }
+  const uint32_t wantCrc = t.crc;
+  const size_t total = (size_t)t.totalSize;
   out->clear();
   try {
     detail::resizeUninitialized(*out, total);  // every block inflates into its own slice; no zero-fill pass on one thread first
@@ -233,7 +229,7 @@ bool decompressGzippedParallel(const uint8_t *data, size_t size, int threads, st
   std::vector<uint32_t> crcs(blocks);
   std::atomic<bool> ok{true};
   parallelFor(blocks, threads, [&](size_t i) {
-    const size_t len = i + 1 == blocks ? lastLen : t.blockSize;
+    const size_t len = t.blockBytes(i);
     z_stream zs;
     std::memset(&zs, 0, sizeof zs);
     if (inflateInit2(&zs, -MAX_WBITS) != Z_OK) { ok = false; return; }
@@ -249,7 +245,7 @@ bool decompressGzippedParallel(const uint8_t *data, size_t size, int threads, st
   });
   uLong crc = crc32(0L, Z_NULL, 0);
   if (ok)
-    for (size_t i = 0; i < blocks; i++) crc = crc32_combine(crc, crcs[i], (z_off_t)(i + 1 == blocks ? lastLen : t.blockSize));
+    for (size_t i = 0; i < blocks; i++) crc = crc32_combine(crc, crcs[i], (z_off_t)t.blockBytes(i));
   if (!ok || (uint32_t)crc != wantCrc) {
     // a damaged table or block: let the serial inflater give the verdict the reference would
     return decompressGzipped(data, size, out);

@@ -113,6 +113,21 @@ void logLine(const char *fmt, ...);
 bool frameBlockMember(size_t size, size_t blockSize, const std::vector<uint32_t> &compressed, uint32_t crc,
                       const std::function<bool(uint8_t *)> &writeBody, std::vector<uint8_t> *out);
 
+// The block table of a member as frameBlockMember writes it, and the trailer's CRC-32.
+struct BlockTable {
+  size_t blockSize = 0;
+  uint64_t totalSize = 0;            // inflated bytes of the whole member
+  std::vector<uint32_t> compressed;  // bytes of each block's deflate data
+  size_t bodyOffset = 0;             // where the deflate data starts
+  uint32_t crc = 0;                  // the trailer's CRC-32 of the inflated bytes
+  uint64_t blockBytes(size_t i) const { return i + 1 == compressed.size() ? totalSize - (uint64_t)i * blockSize : blockSize; }
+};
+// The one parser of the table (spz_gzip.cc), for the host and the device block-parallel inflaters:
+// true when `data` is a gzip member carrying a table those may trust -- it fits the member, agrees with
+// ISIZE, has blocks under 2 GiB and claims no block larger than 1032 times its compressed length plus
+// one.  Reads only the header, the table and the trailer; allocates nothing but t->compressed.
+bool parseBlockTable(const uint8_t *data, size_t size, BlockTable *t);
+
 // What the 16 header bytes and the stream length of an inflated container say (load-spz.cc:548-574),
 // validated before anything is allocated: parseContainer logs and returns false the way the reference
 // fails.  offset / bytes are in stream order: positions, alphas, colors, scales, rotations, sh.
