@@ -155,6 +155,18 @@ int spzb200_encode_device_as(SpzB200Context *ctx, const SpzB200Cloud *in, int32_
 int spzb200_decode_device(SpzB200Context *ctx, const SpzB200Packed *in, int32_t to,
                           SpzB200Cloud *out, void *stream);
 
+/* The cloud an .spz file of `in` gives back: spzb200_encode_device_as(in, from, version) followed by
+ * spzb200_decode_device(to), bit for bit, in one kernel that writes no packed planes (no device scratch).
+ * For training with the quantizer in the loop.  version is SPZB200_STREAM_V3 (smallest-three rotations)
+ * or SPZB200_STREAM_V2 (first-three).  in and out hold DEVICE pointers; out->num_points and out->sh_degree
+ * must equal in's.  Planes need only float alignment (16-byte aligned ones are faster).
+ * Aliasing: each output plane is either exactly its input plane (same pointer: in place) or overlaps no
+ * input plane; output planes do not overlap each other.  Anything else fails with SPZB200_ERR_INVALID.
+ * Every failure is reported before any work is queued, so `out` is untouched then.  Asynchronous on
+ * `stream`, as spzb200_encode_device. */
+int spzb200_quantize_device(SpzB200Context *ctx, const SpzB200Cloud *in /* device */, int32_t from, int32_t to,
+                            int32_t version, SpzB200Cloud *out /* device */, void *stream);
+
 /* ---- host-pointer codec: what the C++ / Python drop-in API calls ----------------------------
  *
  * Same contracts with HOST pointers.  The cloud is cut into contiguous point ranges; each range is

@@ -61,6 +61,7 @@ SIGNATURES = {
     "spzb200_encode_device_as": (C.c_int, [C.c_void_p, C.POINTER(Cloud), C.c_int32, C.c_int32, C.POINTER(Packed), C.c_void_p]),
     "spzb200_encode_host_as": (C.c_int, [C.c_void_p, C.POINTER(Cloud), C.c_int32, C.c_int32, C.POINTER(Packed), C.POINTER(Timings)]),
     "spzb200_decode_device": (C.c_int, [C.c_void_p, C.POINTER(Packed), C.c_int32, C.POINTER(Cloud), C.c_void_p]),
+    "spzb200_quantize_device": (C.c_int, [C.c_void_p, C.POINTER(Cloud), C.c_int32, C.c_int32, C.c_int32, C.POINTER(Cloud), C.c_void_p]),
     "spzb200_encode_host": (C.c_int, [C.c_void_p, C.POINTER(Cloud), C.c_int32, C.POINTER(Packed), C.POINTER(Timings)]),
     "spzb200_decode_host": (C.c_int, [C.c_void_p, C.POINTER(Packed), C.c_int32, C.POINTER(Cloud), C.POINTER(Timings)]),
     "spzb200_encode_ply_device": (C.c_int, [C.c_void_p, C.POINTER(PlyRows), C.c_int32, C.POINTER(Packed), C.c_void_p]),

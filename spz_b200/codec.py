@@ -340,6 +340,28 @@ class Context:
         N.check(N.lib().spzb200_decode_device(self._h, C.byref(ps), int(to), C.byref(cs), C.c_void_p(self._stream_handle(stream))))
         return out
 
+    def quantize_device(self, cloud: CloudPlanes, frm: int = 0, to: Optional[int] = None, version: int = 3,
+                        out: Optional[CloudPlanes] = None, stream=None) -> CloudPlanes:
+        """decode_device(encode_device(cloud, frm, version=version), to), bit for bit, in one kernel that writes no
+        packed planes (spzb200_quantize_device): the cloud an .spz file of `cloud` gives back.  to=None means
+        to=frm.  out=cloud runs in place; any other overlap between the planes of `out` and `cloud` is refused.
+        Wrong plane sizes, an SH degree outside 0..3, a version other than 2 or 3 and overlaps raise
+        CodecError(ERR_INVALID) and leave `out` untouched."""
+        if to is None:
+            to = frm
+        if cloud.sh_degree not in SH_DIM:
+            raise N.CodecError(N.ERR_INVALID, f"quantize_device: sh_degree {cloud.sh_degree} not in 0..3")
+        if out is None:
+            out = alloc_cloud(cloud.n, cloud.sh_degree, device=cloud.positions.device)
+        try:
+            cs, os_ = _cloud_struct(cloud, True), _cloud_struct(out, True)
+        except (TypeError, ValueError) as e:
+            raise N.CodecError(N.ERR_INVALID, f"quantize_device: {e}") from e
+        N.check(N.lib().spzb200_quantize_device(self._h, C.byref(cs), int(frm), int(to), int(version), C.byref(os_),
+                                                C.c_void_p(self._stream_handle(stream))))
+        out.antialiased = cloud.antialiased
+        return out
+
     # ---- .spz files of device-resident clouds (the deflate stage on the device) ------------------
     def _take_bytes(self, rc: int, out: C.c_void_p, size: C.c_size_t) -> bytes:
         N.check(rc)
@@ -490,6 +512,43 @@ class Context:
         N.check(N.lib().spzb200_unpack_gather_device(self._h, C.byref(ps), None if indices is None else C.c_void_p(indices.data_ptr()), count, cp,
                                                      C.c_void_p(out.data_ptr()), C.c_void_p(self._stream_handle(stream))))
         return out
+
+
+_straight_through_fn = None
+
+
+def _straight_through():
+    """The autograd.Function behind quantize_straight_through, defined on first use (torch is imported lazily)."""
+    global _straight_through_fn
+    if _straight_through_fn is None:
+        import torch
+
+        class QuantizeStraightThrough(torch.autograd.Function):
+            @staticmethod
+            def forward(fctx, codec_ctx, n, sh_degree, antialiased, frm, version, *planes):
+                cloud = CloudPlanes(n, sh_degree, *planes, antialiased=antialiased)
+                out = codec_ctx.quantize_device(cloud, frm, frm, version)
+                # an output plane carries a gradient only when its input plane asks for one
+                fctx.mark_non_differentiable(*[o for o, p in zip(out.planes(), planes) if p is None or not p.requires_grad])
+                return out.planes()
+
+            @staticmethod
+            def backward(fctx, *grads):
+                return (None,) * 6 + tuple(g if need else None for need, g in zip(fctx.needs_input_grad[6:], grads))
+
+        _straight_through_fn = QuantizeStraightThrough
+    return _straight_through_fn
+
+
+def quantize_straight_through(ctx: Context, cloud: CloudPlanes, frm: int = 0, version: int = 3) -> CloudPlanes:
+    """ctx.quantize_device(cloud, frm, frm, version) as an autograd op with the straight-through estimator: the
+    forward pass is the codec's round trip, and the backward pass hands each plane's incoming gradient to the
+    matching input plane unchanged, as if the round trip were the identity.  No gradient flows through the
+    quantizer's steps (their true derivative is zero almost everywhere); this is the usual way to fine-tune a
+    cloud with the quantizer in the loop.  The output is in the input's frame (to = frm), so the identity is
+    the right Jacobian for the flips too.  Returns new planes; `cloud` is not modified."""
+    planes = _straight_through().apply(ctx, cloud.n, cloud.sh_degree, cloud.antialiased, int(frm), int(version), *cloud.planes())
+    return CloudPlanes(cloud.n, cloud.sh_degree, *planes, antialiased=cloud.antialiased)
 
 
 RECORD_BYTES = 65      # sizeof(PackedGaussian), load-spz.h:28-37

@@ -1303,6 +1303,73 @@ int spzb200_decode_device(SpzB200Context *ctx, const SpzB200Packed *in, int32_t 
   return SPZB200_OK;
 }
 
+namespace {
+// An output plane may be its own input plane (in place).  Any other overlap of an output plane with an
+// input or another output plane would make the result depend on the order the CTAs run in.
+int checkQuantizeOverlap(const SpzB200Cloud &in, const SpzB200Cloud &out, const char *who) {
+  size_t per[6];
+  floatPlaneBytes(shDimOf(in.sh_degree), per);
+  const float *ip[6] = {in.positions, in.scales, in.rotations, in.alphas, in.colors, in.sh};
+  const float *op[6] = {out.positions, out.scales, out.rotations, out.alphas, out.colors, out.sh};
+  auto overlap = [&](const float *a, size_t aBytes, const float *b, size_t bBytes) {
+    const uintptr_t x = reinterpret_cast<uintptr_t>(a), y = reinterpret_cast<uintptr_t>(b);
+    return x < y + bBytes && y < x + aBytes;
+  };
+  for (int i = 0; i < 6; i++) {
+    const size_t bi = per[i] * (size_t)out.num_points;
+    if (bi == 0) continue;
+    for (int j = 0; j < 6; j++) {
+      const size_t bj = per[j] * (size_t)out.num_points;
+      if (bj == 0) continue;
+      if (overlap(op[i], bi, ip[j], bj) && !(i == j && op[i] == ip[j]))
+        return fail(SPZB200_ERR_INVALID, "%s: output plane %d overlaps input plane %d other than exactly (in place)", who, i, j);
+      if (j != i && overlap(op[i], bi, op[j], bj))
+        return fail(SPZB200_ERR_INVALID, "%s: output planes %d and %d overlap", who, i, j);
+    }
+  }
+  return SPZB200_OK;
+}
+}  // namespace
+
+int spzb200_quantize_device(SpzB200Context *ctx, const SpzB200Cloud *in, int32_t from, int32_t to, int32_t version,
+                            SpzB200Cloud *out, void *stream) {
+  const char *who = "spzb200_quantize_device";
+  if (!ctx) return fail(SPZB200_ERR_INVALID, "%s: null context", who);
+  if (version != SPZB200_STREAM_V2 && version != SPZB200_STREAM_V3)
+    return fail(SPZB200_ERR_INVALID, "%s: the encoder writes stream version 2 or 3, not %d", who, version);
+  int rc = checkCloud(in, who);
+  if (rc) return rc;
+  if (!out) return fail(SPZB200_ERR_INVALID, "%s: null out", who);
+  rc = checkCloud(out, who);
+  if (rc) return rc;
+  if (out->num_points != in->num_points || out->sh_degree != in->sh_degree)
+    return fail(SPZB200_ERR_INVALID, "%s: out holds %lld points of SH degree %d, in %lld of degree %d", who, (long long)out->num_points,
+                out->sh_degree, (long long)in->num_points, in->sh_degree);
+  if (from < 0 || from > 8) return fail(SPZB200_ERR_INVALID, "%s: coordinate system %d", who, from);
+  if (to < 0 || to > 8) return fail(SPZB200_ERR_INVALID, "%s: coordinate system %d", who, to);
+  rc = checkQuantizeOverlap(*in, *out, who);
+  if (rc) return rc;
+  spzb200::QuantizeArgs a;
+  a.positions = in->positions; a.scales = in->scales; a.rotations = in->rotations;
+  a.alphas = in->alphas; a.colors = in->colors; a.sh = in->sh;
+  a.oPositions = out->positions; a.oScales = out->scales; a.oRotations = out->rotations;
+  a.oAlphas = out->alphas; a.oColors = out->colors; a.oSh = out->sh;
+  a.n = in->num_points;
+  a.shDim = shDimOf(in->sh_degree);
+  a.version = version;
+  const spzb200::m::FlipBits f = spzb200::m::make_flip_bits(from, SPZB200_COORD_RUB);
+  a.flipP = f.p; a.flipQ = f.q; a.flipSh = f.sh;
+  const spzb200::m::FlipBits g = spzb200::m::make_flip_bits(SPZB200_COORD_RUB, to);
+  a.oFlipP = g.p; a.oFlipQ = g.q; a.oFlipSh = g.sh;
+  a.alphaThresholds = ctx->dThr;
+  a.tables = ctx->dLut;
+  CU(cudaSetDevice(ctx->device));
+  int launches = 0;
+  CU(spzb200::launchQuantize(a, planOf(ctx), (cudaStream_t)stream, &launches));
+  ctx->kernelLaunches += launches;
+  return SPZB200_OK;
+}
+
 int spzb200_encode_host(SpzB200Context *ctx, const SpzB200Cloud *in, int32_t from,
                         SpzB200Packed *out, SpzB200Timings *timings) {
   return spzb200_encode_host_as(ctx, in, from, SPZB200_STREAM_V3, out, timings);

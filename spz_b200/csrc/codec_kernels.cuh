@@ -34,6 +34,21 @@ struct DecodeArgs {
 
 constexpr int kDecodeTableFloats = 1024;
 
+// GaussianCloud planes -> the planes launchDecode(launchEncode(x)) gives back, both device-resident,
+// without packed planes in between (quantize_kernels.cu).  An output plane may be its input plane (in
+// place); no other overlap is allowed.  Positions use 12 fractional bits, as the encoder writes them.
+struct QuantizeArgs {
+  const float *positions, *scales, *rotations, *alphas, *colors, *sh;
+  float *oPositions, *oScales, *oRotations, *oAlphas, *oColors, *oSh;
+  long long n;
+  int shDim;
+  int version;                       // 3: smallest-three rotations; 2: first-three (as EncodeArgs)
+  uint32_t flipP, flipQ, flipSh;     // sign-bit sets of coordinateConverter(from, RUB)
+  uint32_t oFlipP, oFlipQ, oFlipSh;  // sign-bit sets of coordinateConverter(RUB, to)
+  const float *alphaThresholds;      // as EncodeArgs
+  const float *tables;               // as DecodeArgs
+};
+
 // PLY vertex records (row-major, `width` floats per vertex) -> PackedGaussians planes, both
 // device-resident: loadSplatFromPly's column shuffle (load-spz.cc:808-838) fused with packGaussians.
 struct PlyEncodeArgs {
@@ -108,6 +123,8 @@ cudaError_t launchEncode(const EncodeArgs &a, const LaunchPlan &plan, cudaStream
                          int *launches);
 cudaError_t launchDecode(const DecodeArgs &a, const LaunchPlan &plan, cudaStream_t stream,
                          int *launches);
+// One launch (none for n = 0); uses plan.pdl only.
+cudaError_t launchQuantize(const QuantizeArgs &a, const LaunchPlan &plan, cudaStream_t stream, int *launches);
 
 cudaError_t launchEncodePly(const PlyEncodeArgs &a, const LaunchPlan &plan, cudaStream_t stream, int *launches);
 cudaError_t launchDecodePly(const PlyDecodeArgs &a, const LaunchPlan &plan, cudaStream_t stream, int *launches);
