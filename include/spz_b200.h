@@ -303,7 +303,7 @@ int spzb200_gzip_table_info(const uint8_t *bytes, size_t size, uint64_t *inflate
  * vouch for a block, the host inflater produces the bytes.  *on_device (may be NULL) = 1 when the device
  * produced them.  Synchronous, after earlier work on `stream`.  A member without the table fails with
  * SPZB200_ERR_INVALID before anything is allocated; after a failure the contents of `out` are undefined.
- * Device scratch: the compressed body. */
+ * Device scratch: the compressed body and 24 bytes per table block. */
 int spzb200_gunzip_device(SpzB200Context *ctx, const uint8_t *bytes, size_t size, uint8_t *out,
                           size_t out_capacity, size_t *out_size, int32_t *on_device, void *stream);
 
@@ -322,6 +322,47 @@ int spzb200_gunzip_device(SpzB200Context *ctx, const uint8_t *bytes, size_t size
  * on the host route.  Returns when `out` is complete. */
 int spzb200_load_spz_device(SpzB200Context *ctx, const uint8_t *bytes /* host */, size_t size, int32_t to,
                             SpzB200Cloud *out /* device */, int32_t *antialiased, void *stream);
+
+/* ---- batches of .spz files of device-resident clouds (DESIGN.md section 10c) ------------------
+ *
+ * One call for many files: the table blocks of all members go to one inflate launch, the segments of all
+ * inputs to one set of deflate launches, and the planes of all files to one plane-move launch, so small
+ * files share the GPU instead of each paying a launch and its latency.  Entry i of every result is
+ * exactly what the single-file call gives for input i alone.  Synchronous, after earlier work on
+ * `stream`; device scratch is allocated and freed on `stream` and peaks at the sum over the files of
+ * what the single call uses.  count may be 0 (nothing is done). */
+
+/* spzb200_gzip_device of each of data[0..count) (device; sizes[i] bytes): out[i], out_size[i] are what
+ * spzb200_gzip_device writes for input i.  Release each out[i] with spzb200_free.  All or nothing: on
+ * failure every out[i] is NULL. */
+int spzb200_gzip_device_batch(SpzB200Context *ctx, const uint8_t *const *data /* device */, const size_t *sizes, int32_t count,
+                              uint8_t **out, size_t *out_size, void *stream);
+
+/* spzb200_save_spz_device of each of clouds[0..count) (device planes), all from coordinate system
+ * `from`; antialiased[i] is cloud i's header flag (antialiased may be NULL: none is).  Every cloud is
+ * checked before anything is queued.  All or nothing: on failure every out[i] is NULL. */
+int spzb200_save_spz_device_batch(SpzB200Context *ctx, const SpzB200Cloud *clouds /* device */, int32_t count, int32_t from,
+                                  const int32_t *antialiased, uint8_t **out, size_t *out_size, void *stream);
+
+/* spzb200_gunzip_device of each member bytes[i] (host; sizes[i] bytes) into out[i] (device,
+ * out_capacity[i] bytes): status[i], out_size[i], on_device[i] (on_device may be NULL) and the bytes are
+ * what spzb200_gunzip_device gives for member i alone.  A member the device cannot vouch for is inflated
+ * by the host inflater on its own; its neighbours are not affected.  Returns SPZB200_ERR_INVALID when any
+ * member failed, OK otherwise; a CUDA or allocation failure ends the call with its code. */
+int spzb200_gunzip_device_batch(SpzB200Context *ctx, const uint8_t *const *bytes /* host */, const size_t *sizes, int32_t count,
+                                uint8_t *const *out /* device */, const size_t *out_capacity, size_t *out_size, int32_t *on_device,
+                                int32_t *status, void *stream);
+
+/* spzb200_load_spz_device of each file bytes[i] (host; sizes[i] bytes) into out[i] (device planes sized
+ * by spzb200_spz_info), all to coordinate system `to`; antialiased[i] (antialiased may be NULL) receives
+ * file i's header flag.  Per file, the route and the verdict are those of spzb200_load_spz_device: the
+ * members with table blocks under 1 MiB whose headers agree with their out[i] are inflated together on
+ * the device, every other file and every member the device cannot vouch for takes the host route.  A file
+ * that fails has status[i] = SPZB200_ERR_INVALID and out[i] untouched; the others are complete.  Returns
+ * SPZB200_ERR_INVALID when any file failed, OK otherwise; a CUDA or allocation failure ends the call with
+ * its code. */
+int spzb200_load_spz_device_batch(SpzB200Context *ctx, const uint8_t *const *bytes /* host */, const size_t *sizes, int32_t count,
+                                  int32_t to, SpzB200Cloud *out /* device */, int32_t *antialiased, int32_t *status, void *stream);
 
 /* Point range [*begin, *end) of shard `index` out of `num_shards` over n gaussians of the given
  * SH degree.  Boundaries are multiples of the kernel tile, so every shard but the last runs

@@ -83,6 +83,12 @@ SIGNATURES = {
     "spzb200_gzip_table_info": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(C.c_uint64), C.POINTER(C.c_int64)]),
     "spzb200_gunzip_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t),
                                         C.POINTER(C.c_int32), C.c_void_p]),
+    "spzb200_gzip_device_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "spzb200_save_spz_device_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "spzb200_gunzip_device_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                              C.c_void_p, C.c_void_p]),
+    "spzb200_load_spz_device_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                C.c_void_p]),
     "spzb200_shard_range": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "spzb200_tile_gaussians": (C.c_int32, [C.c_int32]),
     "spzb200_flip_bits": (None, [C.c_int32, C.c_int32, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
@@ -137,9 +143,10 @@ def last_error() -> str:
 
 
 class CodecError(RuntimeError):
-    def __init__(self, code: int, message: str):
+    def __init__(self, code: int, message: str, failed=()):
         super().__init__(f"spz_b200 error {code}: {message}")
         self.code = code
+        self.failed = list(failed)  # batch calls: the indices of the inputs that failed
 
 
 def check(rc: int) -> None:

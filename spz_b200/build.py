@@ -18,7 +18,7 @@ CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_lib")
 LIB = os.path.join(OUT_DIR, "libspz_b200.so")
 
-CUDA_SOURCES = ["codec_kernels.cu", "ply_kernels.cu", "pergaussian_kernels.cu", "gather_kernels.cu", "deflate_kernels.cu", "inflate_kernels.cu", "quantize_kernels.cu", "cabi.cu"]
+CUDA_SOURCES = ["codec_kernels.cu", "ply_kernels.cu", "pergaussian_kernels.cu", "gather_kernels.cu", "deflate_kernels.cu", "inflate_kernels.cu", "quantize_kernels.cu", "move_kernels.cu", "cabi.cu"]
 CXX_SOURCES = ["spz_api.cc", "spz_ply.cc", "spz_gzip.cc"]
 
 NVCC_FLAGS = [

@@ -416,6 +416,105 @@ class Context:
         out.antialiased = bool(aa.value)
         return out, out.antialiased
 
+    # ---- batches of .spz files: one inflate or deflate launch per batch (DESIGN.md section 10c) -------
+    @staticmethod
+    def _host_blobs(blobs):
+        bufs = [np.frombuffer(b, np.uint8) if not isinstance(b, np.ndarray) else np.ascontiguousarray(b, np.uint8) for b in blobs]
+        ptrs = (C.c_void_p * max(len(bufs), 1))(*[b.ctypes.data for b in bufs])
+        sizes = (C.c_size_t * max(len(bufs), 1))(*[b.size for b in bufs])
+        return bufs, ptrs, sizes
+
+    def _take_all(self, rc: int, outs, sizes, count: int):
+        N.check(rc)
+        try:
+            return [C.string_at(outs[i], sizes[i]) for i in range(count)]
+        finally:
+            for i in range(count):
+                N.lib().spzb200_free(C.c_void_p(outs[i]))
+
+    @staticmethod
+    def _batch_failed(what: str, status, count: int):
+        failed = [i for i in range(count) if status[i] != N.OK]
+        raise N.CodecError(N.ERR_INVALID, f"{what}: inputs {failed} failed ({N.last_error()})", failed)
+
+    def gzip_device_batch(self, tensors, stream=None) -> list:
+        """gzip_device of each contiguous uint8 CUDA tensor, every segment of the batch in one set of deflate
+        launches (spzb200_gzip_device_batch).  Entry i equals gzip_device(tensors[i]) byte for byte."""
+        k = len(tensors)
+        ptrs = (C.c_void_p * max(k, 1))(*[_ptr(t, "u1", t.numel(), True, f"tensors[{i}]") or None for i, t in enumerate(tensors)])
+        sizes = (C.c_size_t * max(k, 1))(*[t.numel() for t in tensors])
+        outs, got = (C.c_void_p * max(k, 1))(), (C.c_size_t * max(k, 1))()
+        rc = N.lib().spzb200_gzip_device_batch(self._h, ptrs, sizes, k, outs, got, C.c_void_p(self._stream_handle(stream)))
+        return self._take_all(rc, outs, got, k)
+
+    def save_spz_device_batch(self, clouds, frm: int = 0, antialiased=False, stream=None) -> list:
+        """save_spz_device of each cloud (spzb200_save_spz_device_batch): one plane-move launch and one set of
+        deflate launches for the batch.  antialiased: one flag for all, or one per cloud."""
+        k = len(clouds)
+        flags = list(antialiased) if isinstance(antialiased, (list, tuple)) else [antialiased] * k
+        if len(flags) != k:
+            raise N.CodecError(N.ERR_INVALID, f"save_spz_device_batch: {len(flags)} antialiased flags for {k} clouds")
+        structs = (N.Cloud * max(k, 1))(*[_cloud_struct(c, True) for c in clouds])
+        aa = (C.c_int32 * max(k, 1))(*[int(bool(f)) for f in flags])
+        outs, got = (C.c_void_p * max(k, 1))(), (C.c_size_t * max(k, 1))()
+        rc = N.lib().spzb200_save_spz_device_batch(self._h, structs, k, int(frm), aa, outs, got, C.c_void_p(self._stream_handle(stream)))
+        return self._take_all(rc, outs, got, k)
+
+    def gunzip_device_batch(self, blobs, outs=None, stream=None) -> list:
+        """gunzip_device of each block-table gzip member (spzb200_gunzip_device_batch): every table block of the
+        batch in one inflate launch -> [(uint8 CUDA tensor, on_device)].  `outs`, if given, holds one
+        contiguous uint8 CUDA tensor per member.  Raises CodecError(ERR_INVALID) whose `failed` lists the
+        members that failed; the others' outputs are complete then."""
+        import torch
+        bufs, ptrs, sizes = self._host_blobs(blobs)
+        k = len(bufs)
+        if outs is None:
+            outs = []
+            for b in bufs:
+                try:
+                    n = gzip_table_info(b)[0]
+                except N.CodecError:
+                    n = 0  # the call gives this member's verdict
+                outs.append(torch.empty(n, dtype=torch.uint8, device=f"cuda:{self.device}"))
+        dst = (C.c_void_p * max(k, 1))(*[_ptr(o, "u1", o.numel(), True, f"outs[{i}]") for i, o in enumerate(outs)])
+        cap = (C.c_size_t * max(k, 1))(*[o.numel() for o in outs])
+        got, on_dev, status = (C.c_size_t * max(k, 1))(), (C.c_int32 * max(k, 1))(), (C.c_int32 * max(k, 1))()
+        rc = N.lib().spzb200_gunzip_device_batch(self._h, ptrs, sizes, k, dst, cap, got, on_dev, status,
+                                                 C.c_void_p(self._stream_handle(stream)))
+        if rc == N.ERR_INVALID and any(status[i] for i in range(k)):
+            self._batch_failed("gunzip_device_batch", status, k)
+        N.check(rc)
+        return [(outs[i][:got[i]], bool(on_dev[i])) for i in range(k)]
+
+    def load_spz_device_batch(self, blobs, to: int = 0, device=None, outs=None, stream=None) -> list:
+        """load_spz_device of each .spz file (spzb200_load_spz_device_batch): the device-route files' table
+        blocks in one inflate launch and their planes in one move launch -> [(CloudPlanes, antialiased)].
+        `outs`, if given, holds one CloudPlanes per file sized by spz_info.  Raises CodecError(ERR_INVALID)
+        whose message and `failed` list the files that failed; their outs are untouched, the others' complete."""
+        bufs, ptrs, sizes = self._host_blobs(blobs)
+        k = len(bufs)
+        if outs is None:
+            dev = device if device is not None else f"cuda:{self.device}"
+            outs = []
+            for b in bufs:
+                try:
+                    n, deg = spz_info(b)
+                except N.CodecError:
+                    n, deg = 0, 0  # the call gives this file's verdict
+                outs.append(alloc_cloud(n, deg, device=dev))
+        structs = (N.Cloud * max(k, 1))(*[_cloud_struct(o, True) for o in outs])
+        aa, status = (C.c_int32 * max(k, 1))(), (C.c_int32 * max(k, 1))()
+        rc = N.lib().spzb200_load_spz_device_batch(self._h, ptrs, sizes, k, int(to), structs, aa, status,
+                                                   C.c_void_p(self._stream_handle(stream)))
+        if rc in (N.OK, N.ERR_INVALID):
+            for i, o in enumerate(outs):
+                if status[i] == N.OK:
+                    o.antialiased = bool(aa[i])
+        if rc == N.ERR_INVALID and any(status[i] for i in range(k)):
+            self._batch_failed("load_spz_device_batch", status, k)
+        N.check(rc)
+        return [(o, o.antialiased) for o in outs]
+
     # ---- fused PLY-rows encoder ---------------------------------------------------------------
     def encode_ply_device(self, rows, n: int, names, sh_degree: int, frm: int = 0, out: Optional[PackedPlanes] = None, stream=None):
         if out is None:

@@ -13,6 +13,7 @@
 #endif
 
 #include <algorithm>
+#include <array>
 #include <chrono>
 #include <cmath>
 #include <cstdarg>
@@ -32,6 +33,7 @@
 
 #include "../../include/spz_b200.h"
 #include "../../include/spz_b200/spz.hpp"
+#include "batch_plan.hpp"
 #include "codec_kernels.cuh"
 #include "codec_math.cuh"
 #include "deflate_format.cuh"
@@ -1995,121 +1997,213 @@ struct DeviceScratch {
 
 size_t deflateBodyBytes(size_t size) { return size + 16 * spzb200::dfl::segmentCount(size) + 16; }
 
-// `bytes` between pageable host memory and the device, stream-ordered after earlier work on `stream`, in
-// pieces through two of the context's pinned bounce buffers: the DMA of one piece overlaps the host copy
-// of the next (a pageable copy of a whole compressed body ran at ~2 GB/s on a B200 host).  Synchronous.
-int bouncedCopy(SpzB200Context *ctx, void *dst, const void *src, size_t bytes, cudaMemcpyKind kind, cudaStream_t stream) {
+struct HostSpan {
+  const uint8_t *p;
+  size_t n;
+};
+
+// The spans, end to end, from pageable host memory to dst on the device, stream-ordered after earlier
+// work on `stream`, in pieces through two of the context's pinned bounce buffers: the DMA of one piece
+// overlaps the host copy of the next (a pageable copy of a whole compressed body ran at ~2 GB/s on a B200
+// host).  Synchronous.
+int bouncedUpload(SpzB200Context *ctx, uint8_t *dst, const std::vector<HostSpan> &src, cudaStream_t stream) {
   constexpr size_t kPiece = (size_t)8 << 20;
-  const bool down = kind == cudaMemcpyDeviceToHost;
   for (int k = 0; k < 2; k++) {
     Stage &s = ctx->stage[k];
-    const int rc = down ? ensureBounce(s.hOut, s.hOutCap, kPiece) : ensureBounce(s.hIn, s.hInCap, kPiece);
+    const int rc = ensureBounce(s.hIn, s.hInCap, kPiece);
     if (rc) return rc;
   }
-  uint8_t *to = static_cast<uint8_t *>(dst);
-  const uint8_t *from = static_cast<const uint8_t *>(src);
+  size_t bytes = 0;
+  for (const HostSpan &h : src) bytes += h.n;
   const size_t pieces = (bytes + kPiece - 1) / kPiece;
-  auto len = [&](size_t i) { return std::min(kPiece, bytes - i * kPiece); };
-  if (down) {  // queue piece i, then copy piece i - 1 out of its buffer
-    for (size_t i = 0; i <= pieces; i++) {
-      if (i < pieces) {
-        Stage &s = ctx->stage[i & 1];
-        CU(cudaMemcpyAsync(s.hOut, from + i * kPiece, len(i), cudaMemcpyDeviceToHost, stream));
-        CU(cudaEventRecord(s.ev[0], stream));
-      }
-      if (i > 0) {
-        Stage &s = ctx->stage[(i - 1) & 1];
-        CU(cudaEventSynchronize(s.ev[0]));
-        bounceCopy(to + (i - 1) * kPiece, s.hOut, len(i - 1));
-      }
-    }
-    return SPZB200_OK;
-  }
-  // up: wait until the buffer's previous DMA is done, fill it, queue its DMA
-  for (size_t i = 0; i < pieces; i++) {
+  size_t span = 0, at = 0;  // read position: src[span].p + at
+  for (size_t i = 0; i < pieces; i++) {  // wait until the buffer's previous DMA is done, fill it, queue its DMA
     Stage &s = ctx->stage[i & 1];
     if (i >= 2) CU(cudaEventSynchronize(s.ev[0]));
-    bounceCopy(s.hIn, from + i * kPiece, len(i));
-    CU(cudaMemcpyAsync(to + i * kPiece, s.hIn, len(i), cudaMemcpyHostToDevice, stream));
+    const size_t len = std::min(kPiece, bytes - i * kPiece);
+    for (size_t filled = 0; filled < len;) {
+      if (at == src[span].n) {
+        span++;
+        at = 0;
+        continue;
+      }
+      const size_t n = std::min(len - filled, src[span].n - at);
+      bounceCopy(s.hIn + filled, src[span].p + at, n);
+      filled += n;
+      at += n;
+    }
+    CU(cudaMemcpyAsync(dst + i * kPiece, s.hIn, len, cudaMemcpyHostToDevice, stream));
     CU(cudaEventRecord(s.ev[0], stream));
   }
   CU(cudaStreamSynchronize(stream));
   return SPZB200_OK;
 }
 
-// `size` device bytes at src -> one gzip member in *out.  slots: segmentCount * deflateSlotBytes() bytes; body:
-// deflateBodyBytes(size) bytes (may be src itself: the body is written after the last read of src).  Synchronous.
-int gzipDeviceBytes(SpzB200Context *ctx, const uint8_t *src, size_t size, uint8_t *slots, uint8_t *body, DeviceScratch &scratch,
-                    std::vector<uint8_t> *out) {
-  namespace dfl = spzb200::dfl;
-  const size_t segs = dfl::segmentCount(size);
-  uint32_t *segBytes = nullptr;
-  unsigned long long *offsets = nullptr;
-  CU(scratch.alloc(&segBytes, 2 * segs * sizeof(uint32_t)));
-  CU(scratch.alloc(&offsets, (segs + 1) * sizeof(unsigned long long)));
-  uint32_t *segCrc = segBytes + segs;
-  int launches = 0;
-  CU(spzb200::launchDeflate(src, size, slots, segBytes, segCrc, offsets, body, scratch.stream, &launches));
-  ctx->kernelLaunches += launches;
-  std::vector<uint32_t> hostSeg(2 * segs);
-  CU(cudaMemcpyAsync(hostSeg.data(), segBytes, 2 * segs * sizeof(uint32_t), cudaMemcpyDeviceToHost, scratch.stream));
-  CU(cudaStreamSynchronize(scratch.stream));
-  uLong crc = crc32(0L, Z_NULL, 0);
-  const size_t perBlock = dfl::segmentsPerBlock(segs);
-  std::vector<uint32_t> blockBytes((segs + perBlock - 1) / perBlock, 0);
-  for (size_t s = 0; s < segs; s++) {
-    const size_t len = std::min<size_t>(dfl::kSegBytes, size - std::min(size, s * dfl::kSegBytes));
-    crc = crc32_combine(crc, hostSeg[segs + s], (z_off_t)len);
-    blockBytes[s / perBlock] += hostSeg[s];
+// `bytes` between pageable host memory and the device through the bounce buffers (bouncedUpload); the
+// D2H direction queues piece i, then copies piece i - 1 out of its buffer.  Synchronous.
+int bouncedCopy(SpzB200Context *ctx, void *dst, const void *src, size_t bytes, cudaMemcpyKind kind, cudaStream_t stream) {
+  if (kind != cudaMemcpyDeviceToHost)
+    return bouncedUpload(ctx, static_cast<uint8_t *>(dst), {HostSpan{static_cast<const uint8_t *>(src), bytes}}, stream);
+  constexpr size_t kPiece = (size_t)8 << 20;
+  for (int k = 0; k < 2; k++) {
+    Stage &s = ctx->stage[k];
+    const int rc = ensureBounce(s.hOut, s.hOutCap, kPiece);
+    if (rc) return rc;
   }
-  int copyRc = SPZB200_OK;
-  const bool ok = spz::detail::frameBlockMember(size, perBlock * dfl::kSegBytes, blockBytes, (uint32_t)crc,
-                                                [&](uint8_t *dst) {
-                                                  size_t total = 0;
-                                                  for (uint32_t b : blockBytes) total += b;
-                                                  copyRc = bouncedCopy(ctx, dst, body, total, cudaMemcpyDeviceToHost, scratch.stream);
-                                                  return copyRc == SPZB200_OK;
-                                                },
-                                                out);
-  if (copyRc) return copyRc;
-  if (!ok) return fail(SPZB200_ERR_INVALID, "%zu bytes do not fit the gzip block table", size);
+  uint8_t *to = static_cast<uint8_t *>(dst);
+  const uint8_t *from = static_cast<const uint8_t *>(src);
+  const size_t pieces = (bytes + kPiece - 1) / kPiece;
+  auto len = [&](size_t i) { return std::min(kPiece, bytes - i * kPiece); };
+  for (size_t i = 0; i <= pieces; i++) {
+    if (i < pieces) {
+      Stage &s = ctx->stage[i & 1];
+      CU(cudaMemcpyAsync(s.hOut, from + i * kPiece, len(i), cudaMemcpyDeviceToHost, stream));
+      CU(cudaEventRecord(s.ev[0], stream));
+    }
+    if (i > 0) {
+      Stage &s = ctx->stage[(i - 1) & 1];
+      CU(cudaEventSynchronize(s.ev[0]));
+      bounceCopy(to + (i - 1) * kPiece, s.hOut, len(i - 1));
+    }
+  }
   return SPZB200_OK;
 }
 
-// The inflate stage on the device: the table blocks of the member at `bytes` (parsed into t) -> dOut
-// (t.totalSize bytes).  The compressed body crosses PCIe through the bounce buffers, one kernel inflates
-// every block and checksums its slice, and the host combines the CRCs.  *vouched: every block filled
-// its slice exactly and the combined CRC-32 matches the trailer (ISIZE was checked by the parser); when
-// false, dOut holds nothing to use and the host inflater has to give the verdict.  Synchronous.
-int inflateDeviceBytes(SpzB200Context *ctx, const uint8_t *bytes, const spz::detail::BlockTable &t, uint8_t *dOut,
-                       DeviceScratch &scratch, bool *vouched) {
-  *vouched = false;
-  const size_t blocks = t.compressed.size();
-  std::vector<unsigned long long> offset(blocks + 1, 0);
-  for (size_t i = 0; i < blocks; i++) offset[i + 1] = offset[i] + t.compressed[i];
+// A host table to a fresh device allocation of `scratch`, stream-ordered (the host vector must live until
+// the stream is synchronised).
+template <class T>
+int uploadTable(const std::vector<T> &host, T **dev, DeviceScratch &scratch) {
+  CU(scratch.alloc(dev, host.size() * sizeof(T)));
+  if (!host.empty()) CU(cudaMemcpyAsync(*dev, host.data(), host.size() * sizeof(T), cudaMemcpyHostToDevice, scratch.stream));
+  return SPZB200_OK;
+}
+
+// The segments of all inputs (every DeflateSegment of the batch, batch_plan.hpp) deflated in one set of
+// launches, then each input's body framed as one gzip member and handed over to a malloc'd out[i] at once,
+// while its bytes are still in the host's caches.  All or nothing: after a failure every out[i] is NULL.
+// slots: the batch's segment count times deflateSlotBytes(); body: the sum of deflateBodyBytes over the
+// inputs (may hold the inputs themselves: the body is written after the last read of them).  Synchronous.
+int gzipDeviceBatch(SpzB200Context *ctx, const char *who, const uint8_t *const *src, const size_t *sizes, int count, uint8_t *slots,
+                    uint8_t *body, DeviceScratch &scratch, uint8_t **out, size_t *outSize) {
+  namespace dfl = spzb200::dfl;
+  std::vector<unsigned long long> addr(count);
+  std::vector<uint64_t> size64(count);
+  for (int i = 0; i < count; i++) {
+    addr[i] = (unsigned long long)(uintptr_t)src[i];
+    size64[i] = sizes[i];
+  }
+  std::vector<spzb200::DeflateSegment> segs;
+  std::vector<uint64_t> first;
+  spzb200::planDeflate(addr.data(), size64.data(), count, &segs, &first);
+  const size_t total = segs.size();
+  spzb200::DeflateSegment *dSegs = nullptr;
+  uint32_t *segBytes = nullptr;
+  unsigned long long *offsets = nullptr;
+  int rc = uploadTable(segs, &dSegs, scratch);
+  if (rc) return rc;
+  CU(scratch.alloc(&segBytes, 2 * total * sizeof(uint32_t)));
+  CU(scratch.alloc(&offsets, (total + 1) * sizeof(unsigned long long)));
+  uint32_t *segCrc = segBytes + total;
+  int launches = 0;
+  CU(spzb200::launchDeflate(dSegs, total, slots, segBytes, segCrc, offsets, body, scratch.stream, &launches));
+  ctx->kernelLaunches += launches;
+  std::vector<uint32_t> hostSeg(2 * total);
+  CU(cudaMemcpyAsync(hostSeg.data(), segBytes, 2 * total * sizeof(uint32_t), cudaMemcpyDeviceToHost, scratch.stream));
+  CU(cudaStreamSynchronize(scratch.stream));
+  std::vector<uint64_t> bodyStart;
+  std::vector<std::vector<uint32_t>> blockBytes;
+  spzb200::planMemberBodies(hostSeg.data(), first, &bodyStart, &blockBytes);
+  auto undo = [&](int upTo, int rc) {
+    for (int j = 0; j < upTo; j++) {
+      std::free(out[j]);
+      out[j] = nullptr;
+      outSize[j] = 0;
+    }
+    return rc;
+  };
+  int i = 0;
+  try {
+    for (; i < count; i++) {
+      uLong crc = crc32(0L, Z_NULL, 0);
+      for (uint64_t s = first[i]; s < first[i + 1]; s++) crc = crc32_combine(crc, hostSeg[total + s], (z_off_t)segs[s].len);
+      const size_t segCount = first[i + 1] - first[i];
+      std::vector<uint8_t> bytes;
+      int copyRc = SPZB200_OK;
+      const bool ok = spz::detail::frameBlockMember(sizes[i], dfl::segmentsPerBlock(segCount) * dfl::kSegBytes, blockBytes[i], (uint32_t)crc,
+                                                    [&](uint8_t *dst) {
+                                                      copyRc = bouncedCopy(ctx, dst, body + bodyStart[i], bodyStart[i + 1] - bodyStart[i],
+                                                                           cudaMemcpyDeviceToHost, scratch.stream);
+                                                      return copyRc == SPZB200_OK;
+                                                    },
+                                                    &bytes);
+      if (copyRc) return undo(i, copyRc);
+      if (!ok) return undo(i, fail(SPZB200_ERR_INVALID, "%zu bytes do not fit the gzip block table", sizes[i]));
+      const int rc = handOverBytes(true, who, bytes, &out[i], &outSize[i]);
+      if (rc) return undo(i, rc);
+    }
+  } catch (const std::exception &e) {  // a member handed over before the failure must not outlive it
+    return undo(i, fail(SPZB200_ERR_NOMEM, "%s: %s", who, e.what()));
+  }
+  return SPZB200_OK;
+}
+
+// One member of a batched device inflate: its bytes in host memory, its parsed table, where it inflates to.
+struct InflateMember {
+  const uint8_t *bytes;
+  const spz::detail::BlockTable *t;
+  uint8_t *out;
+};
+
+// The inflate stage on the device for members m (every table block of every member in one launch): the
+// compressed bodies cross PCIe through the bounce buffers, one kernel inflates every block and checksums
+// its slice, and the host combines each member's CRCs.  (*vouched)[i]: every block of member i filled its
+// slice exactly and the combined CRC-32 matches the trailer (ISIZE was checked by the parser); when false,
+// its output holds nothing to use and the host inflater has to give the verdict.  Synchronous.
+int inflateDeviceBatch(SpzB200Context *ctx, const std::vector<InflateMember> &m, DeviceScratch &scratch, std::vector<char> *vouched) {
+  const int count = (int)m.size();
+  vouched->assign(count, 0);
+  std::vector<uint64_t> blockSize(count), total(count), nBlocks(count);
+  std::vector<uint32_t> compressed;
+  std::vector<unsigned long long> outAddr(count);
+  for (int i = 0; i < count; i++) {
+    blockSize[i] = m[i].t->blockSize;
+    total[i] = m[i].t->totalSize;
+    nBlocks[i] = m[i].t->compressed.size();
+    compressed.insert(compressed.end(), m[i].t->compressed.begin(), m[i].t->compressed.end());
+    outAddr[i] = (unsigned long long)(uintptr_t)m[i].out;
+  }
+  std::vector<spzb200::InflateBlock> blocks;
+  std::vector<uint64_t> first, bodyStart;
+  spzb200::planInflate(count, blockSize.data(), total.data(), nBlocks.data(), compressed.data(), outAddr.data(), &blocks, &first, &bodyStart);
+  const size_t nb = blocks.size();
+  if (nb == 0) return SPZB200_OK;
   uint8_t *body = nullptr;
-  unsigned long long *dOffset = nullptr;
+  spzb200::InflateBlock *dBlocks = nullptr;
   uint32_t *dCrc = nullptr;
-  CU(scratch.alloc(&body, offset[blocks]));
-  CU(scratch.alloc(&dOffset, (blocks + 1) * sizeof(unsigned long long)));
-  CU(scratch.alloc(&dCrc, 2 * blocks * sizeof(uint32_t)));
-  int32_t *dStatus = reinterpret_cast<int32_t *>(dCrc + blocks);
-  CU(cudaMemcpyAsync(dOffset, offset.data(), (blocks + 1) * sizeof(unsigned long long), cudaMemcpyHostToDevice, scratch.stream));
-  const int rc = bouncedCopy(ctx, body, bytes + t.bodyOffset, offset[blocks], cudaMemcpyHostToDevice, scratch.stream);
+  CU(scratch.alloc(&body, bodyStart[count]));
+  int rc = uploadTable(blocks, &dBlocks, scratch);
+  if (rc) return rc;
+  CU(scratch.alloc(&dCrc, 2 * nb * sizeof(uint32_t)));
+  int32_t *dStatus = reinterpret_cast<int32_t *>(dCrc + nb);
+  std::vector<HostSpan> spans(count);
+  for (int i = 0; i < count; i++) spans[i] = HostSpan{m[i].bytes + m[i].t->bodyOffset, (size_t)(bodyStart[i + 1] - bodyStart[i])};
+  rc = bouncedUpload(ctx, body, spans, scratch.stream);
   if (rc) return rc;
   int warps = 0;
-  CU(spzb200::launchInflate(body, dOffset, (long long)blocks, t.blockSize, t.totalSize, dOut, dCrc, dStatus, ctx->smCount,
-                            scratch.stream, &warps));
+  CU(spzb200::launchInflate(body, dBlocks, (long long)nb, dCrc, dStatus, ctx->smCount, scratch.stream, &warps));
   ctx->kernelLaunches += 1;
-  std::vector<uint32_t> result(2 * blocks);
-  CU(cudaMemcpyAsync(result.data(), dCrc, 2 * blocks * sizeof(uint32_t), cudaMemcpyDeviceToHost, scratch.stream));
+  std::vector<uint32_t> result(2 * nb);
+  CU(cudaMemcpyAsync(result.data(), dCrc, 2 * nb * sizeof(uint32_t), cudaMemcpyDeviceToHost, scratch.stream));
   CU(cudaStreamSynchronize(scratch.stream));
-  uLong crc = crc32(0L, Z_NULL, 0);
-  for (size_t i = 0; i < blocks; i++) {
-    if (result[blocks + i] != spzb200::ifl::kOk) return SPZB200_OK;
-    crc = crc32_combine(crc, result[i], (z_off_t)t.blockBytes(i));
+  for (int i = 0; i < count; i++) {
+    uLong crc = crc32(0L, Z_NULL, 0);
+    bool ok = true;
+    for (uint64_t b = first[i]; b < first[i + 1] && ok; b++) {
+      ok = result[nb + b] == spzb200::ifl::kOk;
+      crc = crc32_combine(crc, result[b], (z_off_t)blocks[b].outBytes);
+    }
+    (*vouched)[i] = ok && (uint32_t)crc == m[i].t->crc;
   }
-  *vouched = (uint32_t)crc == t.crc;
   return SPZB200_OK;
 }
 
@@ -2125,6 +2219,180 @@ int guarded(const char *who, uint8_t **out, size_t *outSize, Fn &&fn) {
   }
 }
 
+// spzb200_gzip_device_batch after its argument checks.
+int gzipBatch(SpzB200Context *ctx, const char *who, const uint8_t *const *data, const size_t *sizes, int32_t count, uint8_t **out,
+              size_t *outSize, cudaStream_t stream) {
+  return guarded(who, nullptr, nullptr, [&]() -> int {
+    if (count == 0) return SPZB200_OK;
+    CU(cudaSetDevice(ctx->device));
+    size_t segs = 0, body = 0;
+    for (int i = 0; i < count; i++) {
+      segs += spzb200::dfl::segmentCount(sizes[i]);
+      body += deflateBodyBytes(sizes[i]);
+    }
+    DeviceScratch scratch(stream);
+    uint8_t *slots = nullptr, *dBody = nullptr;
+    CU(scratch.alloc(&slots, segs * spzb200::deflateSlotBytes()));
+    CU(scratch.alloc(&dBody, body));
+    return gzipDeviceBatch(ctx, who, data, sizes, count, slots, dBody, scratch, out, outSize);
+  });
+}
+
+// spzb200_save_spz_device_batch after every cloud has been checked: each cloud's encoder planes go to
+// 16-byte-aligned places of the slots buffer, one move launch writes every header and plane into the
+// containers, and the deflater codes every container's segments in one set of launches.
+int saveBatch(SpzB200Context *ctx, const char *who, const SpzB200Cloud *clouds, int32_t count, int32_t from, const int32_t *antialiased,
+              uint8_t **out, size_t *outSize, cudaStream_t stream) {
+  return guarded(who, nullptr, nullptr, [&]() -> int {
+    if (count == 0) return SPZB200_OK;
+    CU(cudaSetDevice(ctx->device));
+    constexpr size_t kHeader = spz::detail::kContainerHeaderBytes;
+    const int streamOrder[6] = {0, 3, 4, 1, 2, 5};  // container order (positions, alphas, colors, scales, rotations, sh) -> struct order
+    std::vector<std::array<size_t, 6>> plane(count), offset(count);  // struct order; offset within the container
+    std::vector<uint64_t> total(count), aligned(count), bodyBound(count);
+    size_t segs = 0;
+    for (int i = 0; i < count; i++) {
+      bytePlaneBytes(shDimOf(clouds[i].sh_degree), SPZB200_STREAM_V3, plane[i].data());
+      for (size_t &b : plane[i]) b *= (size_t)clouds[i].num_points;
+      total[i] = kHeader;
+      for (int k = 0; k < 6; k++) {
+        offset[i][streamOrder[k]] = total[i];
+        total[i] += plane[i][streamOrder[k]];
+        aligned[i] += alignUp(plane[i][k], 16);
+      }
+      bodyBound[i] = deflateBodyBytes(total[i]);
+      segs += spzb200::dfl::segmentCount(total[i]);
+    }
+    std::vector<uint64_t> planesAt, containerAt;
+    spzb200::planAligned(aligned.data(), count, &planesAt);
+    spzb200::planAligned(bodyBound.data(), count, &containerAt);
+    // Peak scratch: the slots (which first hold the encoder's aligned planes) + the containers (which then hold the bodies).
+    DeviceScratch scratch(stream);
+    uint8_t *slots = nullptr, *containers = nullptr, *headers = nullptr;
+    CU(scratch.alloc(&slots, std::max<size_t>(segs * spzb200::deflateSlotBytes(), planesAt[count])));
+    CU(scratch.alloc(&containers, containerAt[count]));
+    CU(scratch.alloc(&headers, kHeader * count));
+    std::vector<uint8_t> hostHeaders(kHeader * count);
+    std::vector<spzb200::MoveSpan> spans;
+    unsigned long long maxSpan = kHeader;
+    std::vector<const uint8_t *> src(count);
+    std::vector<size_t> sizes(count);
+    for (int i = 0; i < count; i++) {
+      const SpzB200Cloud &c = clouds[i];
+      uint8_t *container = containers + containerAt[i];
+      src[i] = container;
+      sizes[i] = total[i];
+      spz::detail::writeContainerHeader(3, c.num_points, c.sh_degree, antialiased && antialiased[i] != 0, &hostHeaders[kHeader * i]);
+      spans.push_back({(unsigned long long)(uintptr_t)(headers + kHeader * i), (unsigned long long)(uintptr_t)container, kHeader});
+      uint8_t *planes[6], *p = slots + planesAt[i];
+      for (int k = 0; k < 6; k++) {
+        planes[k] = p;
+        p += alignUp(plane[i][k], 16);
+        if (plane[i][k]) {
+          spans.push_back({(unsigned long long)(uintptr_t)planes[k], (unsigned long long)(uintptr_t)(container + offset[i][k]), plane[i][k]});
+          maxSpan = std::max<unsigned long long>(maxSpan, plane[i][k]);
+        }
+      }
+      if (c.num_points == 0) continue;
+      SpzB200Packed packed;
+      std::memset(&packed, 0, sizeof packed);
+      packed.num_points = c.num_points;
+      packed.sh_degree = c.sh_degree;
+      packed.positions = planes[0]; packed.scales = planes[1]; packed.rotations = planes[2];
+      packed.alphas = planes[3]; packed.colors = planes[4]; packed.sh = c.sh_degree ? planes[5] : nullptr;
+      const int erc = spzb200_encode_device_as(ctx, &c, from, SPZB200_STREAM_V3, &packed, stream);
+      if (erc) return erc;
+    }
+    CU(cudaMemcpyAsync(headers, hostHeaders.data(), hostHeaders.size(), cudaMemcpyHostToDevice, stream));
+    spzb200::MoveSpan *dSpans = nullptr;
+    int rc = uploadTable(spans, &dSpans, scratch);
+    if (rc) return rc;
+    int launches = 0;
+    CU(spzb200::launchMoveSpans(dSpans, (long long)spans.size(), maxSpan, stream, &launches));
+    ctx->kernelLaunches += launches;
+    return gzipDeviceBatch(ctx, who, src.data(), sizes.data(), count, slots, containers, scratch, out, outSize);
+  });
+}
+
+// Both save entry points: every cloud is checked before anything is queued.
+int saveSpzDevice(SpzB200Context *ctx, const char *who, const SpzB200Cloud *clouds, int32_t count, int32_t from, const int32_t *antialiased,
+                  uint8_t **out, size_t *outSize, cudaStream_t stream) {
+  if (!ctx) return fail(SPZB200_ERR_INVALID, "%s: null context", who);
+  if (count < 0) return fail(SPZB200_ERR_INVALID, "%s: count %d", who, count);
+  if (count && (!out || !outSize)) return fail(SPZB200_ERR_INVALID, "%s: null output arguments", who);
+  for (int i = 0; i < count; i++) {
+    out[i] = nullptr;
+    outSize[i] = 0;
+  }
+  if (count && !clouds) return fail(SPZB200_ERR_INVALID, "%s: null cloud view", who);
+  for (int i = 0; i < count; i++) {
+    const int rc = checkCloud(&clouds[i], who);
+    if (rc) return rc;
+    if (clouds[i].num_points > std::numeric_limits<int32_t>::max())
+      return fail(SPZB200_ERR_INVALID, "%s: %lld points do not fit the container's 32-bit count", who, (long long)clouds[i].num_points);
+  }
+  if (from < 0 || from > 8) return fail(SPZB200_ERR_INVALID, "%s: coordinate system %d", who, from);
+  return saveBatch(ctx, who, clouds, count, from, antialiased, out, outSize, stream);
+}
+
+// spzb200_gunzip_device_batch after its argument checks: every member with a table is inflated in one
+// device launch; a member the device cannot vouch for is inflated by the host inflater, alone.
+int gunzipBatch(SpzB200Context *ctx, const char *who, const uint8_t *const *bytes, const size_t *sizes, int32_t count, uint8_t *const *out,
+                const size_t *capacity, size_t *outSize, int32_t *onDevice, int32_t *status, cudaStream_t stream) {
+  return guarded(who, nullptr, nullptr, [&]() -> int {
+    std::vector<spz::detail::BlockTable> tables(count);
+    std::vector<InflateMember> members;
+    std::vector<int> index;
+    for (int i = 0; i < count; i++) {
+      outSize[i] = 0;
+      if (onDevice) onDevice[i] = 0;
+      status[i] = SPZB200_OK;
+      const spz::detail::BlockTable &t = tables[i];
+      if (!spz::detail::parseBlockTable(bytes[i], sizes[i], &tables[i]))
+        status[i] = fail(SPZB200_ERR_INVALID, "%s: member %d: not a gzip member with a block table the parallel inflater trusts", who, i);
+      else if (capacity[i] < t.totalSize)
+        status[i] = fail(SPZB200_ERR_INVALID, "%s: member %d: out holds %zu bytes, the member inflates to %llu", who, i, capacity[i],
+                         (unsigned long long)t.totalSize);
+      else {
+        members.push_back({bytes[i], &tables[i], out[i]});
+        index.push_back(i);
+      }
+    }
+    if (!members.empty()) {
+      CU(cudaSetDevice(ctx->device));
+      std::vector<char> vouched;
+      {
+        DeviceScratch scratch(stream);
+        const int rc = inflateDeviceBatch(ctx, members, scratch, &vouched);
+        if (rc) return rc;
+      }
+      for (size_t k = 0; k < members.size(); k++) {
+        const int i = index[k];
+        const spz::detail::BlockTable &t = tables[i];
+        if (!vouched[k]) {  // the host inflater's verdict and bytes; they must fill exactly what the table announced
+          std::vector<uint8_t> host;
+          if (!spz::decompressGzippedParallel(bytes[i], sizes[i], spz::detail::inflateThreads(), &host)) {
+            status[i] = fail(SPZB200_ERR_INVALID, "%s: member %d: not a readable gzip member", who, i);
+            continue;
+          }
+          if (host.size() != t.totalSize) {
+            status[i] = fail(SPZB200_ERR_INVALID, "%s: member %d: inflates to %zu bytes, its block table says %llu", who, i, host.size(),
+                             (unsigned long long)t.totalSize);
+            continue;
+          }
+          const int rc = bouncedCopy(ctx, out[i], host.data(), host.size(), cudaMemcpyHostToDevice, stream);
+          if (rc) return rc;
+        }
+        outSize[i] = (size_t)t.totalSize;
+        if (onDevice) onDevice[i] = vouched[k] ? 1 : 0;
+      }
+    }
+    for (int i = 0; i < count; i++)
+      if (status[i]) return SPZB200_ERR_INVALID;
+    return SPZB200_OK;
+  });
+}
+
 }  // namespace
 
 extern "C" {
@@ -2136,77 +2404,33 @@ int spzb200_gzip_device(SpzB200Context *ctx, const uint8_t *data, size_t size, u
   *out = nullptr;
   *out_size = 0;
   if (!data && size) return fail(SPZB200_ERR_INVALID, "%s: null data", who);
-  return guarded(who, out, out_size, [&]() -> int {
-    CU(cudaSetDevice(ctx->device));
-    DeviceScratch scratch((cudaStream_t)stream);
-    uint8_t *slots = nullptr, *body = nullptr;
-    CU(scratch.alloc(&slots, spzb200::dfl::segmentCount(size) * spzb200::deflateSlotBytes()));
-    CU(scratch.alloc(&body, deflateBodyBytes(size)));
-    std::vector<uint8_t> bytes;
-    const int rc = gzipDeviceBytes(ctx, data, size, slots, body, scratch, &bytes);
-    return rc ? rc : handOverBytes(true, who, bytes, out, out_size);
-  });
+  return gzipBatch(ctx, who, &data, &size, 1, out, out_size, (cudaStream_t)stream);
+}
+
+int spzb200_gzip_device_batch(SpzB200Context *ctx, const uint8_t *const *data, const size_t *sizes, int32_t count, uint8_t **out,
+                              size_t *out_size, void *stream) {
+  const char *who = "spzb200_gzip_device_batch";
+  if (!ctx) return fail(SPZB200_ERR_INVALID, "%s: null context", who);
+  if (count < 0) return fail(SPZB200_ERR_INVALID, "%s: count %d", who, count);
+  if (count && (!out || !out_size)) return fail(SPZB200_ERR_INVALID, "%s: null output arguments", who);
+  for (int i = 0; i < count; i++) {
+    out[i] = nullptr;
+    out_size[i] = 0;
+  }
+  if (count && (!data || !sizes)) return fail(SPZB200_ERR_INVALID, "%s: null data", who);
+  for (int i = 0; i < count; i++)
+    if (!data[i] && sizes[i]) return fail(SPZB200_ERR_INVALID, "%s: null data[%d]", who, i);
+  return gzipBatch(ctx, who, data, sizes, count, out, out_size, (cudaStream_t)stream);
 }
 
 int spzb200_save_spz_device(SpzB200Context *ctx, const SpzB200Cloud *in, int32_t from, int32_t antialiased, uint8_t **out,
                             size_t *out_size, void *stream) {
-  const char *who = "spzb200_save_spz_device";
-  if (!ctx) return fail(SPZB200_ERR_INVALID, "%s: null context", who);
-  if (!out || !out_size) return fail(SPZB200_ERR_INVALID, "%s: null output arguments", who);
-  *out = nullptr;
-  *out_size = 0;
-  int rc = checkCloud(in, who);
-  if (rc) return rc;
-  if (in->num_points > std::numeric_limits<int32_t>::max())
-    return fail(SPZB200_ERR_INVALID, "%s: %lld points do not fit the container's 32-bit count", who, (long long)in->num_points);
-  if (from < 0 || from > 8) return fail(SPZB200_ERR_INVALID, "%s: coordinate system %d", who, from);
-  return guarded(who, out, out_size, [&]() -> int {
-    CU(cudaSetDevice(ctx->device));
-    const cudaStream_t st = (cudaStream_t)stream;
-    const size_t n = (size_t)in->num_points;
-    const int shDim = shDimOf(in->sh_degree);
-    size_t plane[6];  // struct order: positions, scales, rotations, alphas, colors, sh
-    bytePlaneBytes(shDim, SPZB200_STREAM_V3, plane);
-    for (size_t &b : plane) b *= n;
-    // container (stream order: positions, alphas, colors, scales, rotations, sh) after the 16 header bytes
-    const int streamOrder[6] = {0, 3, 4, 1, 2, 5};
-    size_t offset[6], total = spz::detail::kContainerHeaderBytes, aligned = 0;
-    for (int i = 0; i < 6; i++) {
-      offset[streamOrder[i]] = total;
-      total += plane[streamOrder[i]];
-      aligned += alignUp(plane[i], 16);
-    }
-    // Peak scratch: the slots (which first hold the encoder's aligned planes) + the container (which then holds the body).
-    const size_t segs = spzb200::dfl::segmentCount(total);
-    DeviceScratch scratch(st);
-    uint8_t *slots = nullptr, *container = nullptr;
-    CU(scratch.alloc(&slots, std::max(segs * spzb200::deflateSlotBytes(), aligned)));
-    CU(scratch.alloc(&container, deflateBodyBytes(total)));
-    SpzB200Packed packed;
-    std::memset(&packed, 0, sizeof packed);
-    packed.num_points = in->num_points;
-    packed.sh_degree = in->sh_degree;
-    uint8_t *planes[6], *p = slots;
-    for (int i = 0; i < 6; i++) {
-      planes[i] = p;
-      p += alignUp(plane[i], 16);
-    }
-    packed.positions = planes[0]; packed.scales = planes[1]; packed.rotations = planes[2];
-    packed.alphas = planes[3]; packed.colors = planes[4]; packed.sh = shDim ? planes[5] : nullptr;
-    if (n) {
-      const int erc = spzb200_encode_device_as(ctx, in, from, SPZB200_STREAM_V3, &packed, stream);
-      if (erc) return erc;
-    }
-    uint8_t header[spz::detail::kContainerHeaderBytes];
-    spz::detail::writeContainerHeader(3, in->num_points, in->sh_degree, antialiased != 0, header);
-    CU(spzb200::launchStoreBytes16(container, header, st));
-    ctx->kernelLaunches += 1;
-    for (int i = 0; i < 6; i++)
-      if (plane[i]) CU(cudaMemcpyAsync(container + offset[i], planes[i], plane[i], cudaMemcpyDeviceToDevice, st));
-    std::vector<uint8_t> bytes;
-    const int grc = gzipDeviceBytes(ctx, container, total, slots, container, scratch, &bytes);
-    return grc ? grc : handOverBytes(true, who, bytes, out, out_size);
-  });
+  return saveSpzDevice(ctx, "spzb200_save_spz_device", in, 1, from, &antialiased, out, out_size, (cudaStream_t)stream);
+}
+
+int spzb200_save_spz_device_batch(SpzB200Context *ctx, const SpzB200Cloud *clouds, int32_t count, int32_t from, const int32_t *antialiased,
+                                  uint8_t **out, size_t *out_size, void *stream) {
+  return saveSpzDevice(ctx, "spzb200_save_spz_device_batch", clouds, count, from, antialiased, out, out_size, (cudaStream_t)stream);
 }
 
 int spzb200_spz_info(const uint8_t *bytes, size_t size, int64_t *num_points, int32_t *sh_degree) {
@@ -2250,37 +2474,20 @@ int spzb200_gunzip_device(SpzB200Context *ctx, const uint8_t *bytes, size_t size
   const char *who = "spzb200_gunzip_device";
   if (!ctx) return fail(SPZB200_ERR_INVALID, "%s: null context", who);
   if (!bytes || !out || !out_size) return fail(SPZB200_ERR_INVALID, "%s: null argument", who);
-  *out_size = 0;
-  if (on_device) *on_device = 0;
-  return guarded(who, nullptr, nullptr, [&]() -> int {
-    spz::detail::BlockTable t;
-    if (!spz::detail::parseBlockTable(bytes, size, &t))
-      return fail(SPZB200_ERR_INVALID, "%s: not a gzip member with a block table the parallel inflater trusts", who);
-    if (out_capacity < t.totalSize)
-      return fail(SPZB200_ERR_INVALID, "%s: out holds %zu bytes, the member inflates to %llu", who, out_capacity,
-                  (unsigned long long)t.totalSize);
-    CU(cudaSetDevice(ctx->device));
-    const cudaStream_t st = (cudaStream_t)stream;
-    bool vouched = false;
-    {
-      DeviceScratch scratch(st);
-      const int rc = inflateDeviceBytes(ctx, bytes, t, out, scratch, &vouched);
-      if (rc) return rc;
-    }
-    if (!vouched) {  // the host inflater's verdict and bytes; they must fill exactly what the table announced
-      std::vector<uint8_t> host;
-      if (!spz::decompressGzippedParallel(bytes, size, spz::detail::inflateThreads(), &host))
-        return fail(SPZB200_ERR_INVALID, "%s: not a readable gzip member", who);
-      if (host.size() != t.totalSize)
-        return fail(SPZB200_ERR_INVALID, "%s: the member inflates to %zu bytes, its block table says %llu", who, host.size(),
-                    (unsigned long long)t.totalSize);
-      const int rc = bouncedCopy(ctx, out, host.data(), host.size(), cudaMemcpyHostToDevice, st);
-      if (rc) return rc;
-    }
-    *out_size = (size_t)t.totalSize;
-    if (on_device) *on_device = vouched ? 1 : 0;
-    return SPZB200_OK;
-  });
+  int32_t status = SPZB200_OK;
+  return gunzipBatch(ctx, who, &bytes, &size, 1, &out, &out_capacity, out_size, on_device, &status, (cudaStream_t)stream);
+}
+
+int spzb200_gunzip_device_batch(SpzB200Context *ctx, const uint8_t *const *bytes, const size_t *sizes, int32_t count, uint8_t *const *out,
+                                const size_t *out_capacity, size_t *out_size, int32_t *on_device, int32_t *status, void *stream) {
+  const char *who = "spzb200_gunzip_device_batch";
+  if (!ctx) return fail(SPZB200_ERR_INVALID, "%s: null context", who);
+  if (count < 0) return fail(SPZB200_ERR_INVALID, "%s: count %d", who, count);
+  if (count == 0) return SPZB200_OK;
+  if (!bytes || !sizes || !out || !out_capacity || !out_size || !status) return fail(SPZB200_ERR_INVALID, "%s: null argument", who);
+  for (int i = 0; i < count; i++)
+    if (!bytes[i] || (!out[i] && out_capacity[i])) return fail(SPZB200_ERR_INVALID, "%s: null bytes[%d] or out[%d]", who, i, i);
+  return gunzipBatch(ctx, who, bytes, sizes, count, out, out_capacity, out_size, on_device, status, (cudaStream_t)stream);
 }
 
 }  // extern "C"
@@ -2294,44 +2501,8 @@ namespace {
 // profiles/r4_device_inflate_timing_unrouted.jsonl; DESIGN.md section 10b).
 constexpr size_t kDeviceLoadMaxBlock = (size_t)1 << 20;
 
-// load_spz_device for a member with a block table: the container is inflated on the device, its planes
-// are moved to 16-byte-aligned places and decoded.  *taken = false (and `out` untouched) whenever this
-// route cannot finish the call -- the header or the table disagree with `out`, the device cannot vouch
-// for a block, an allocation fails -- and the caller then runs the host route, whose verdict is the
-// call's.  After *taken = true the result is the call's result.
-int loadSpzDeviceInflated(SpzB200Context *ctx, const uint8_t *bytes, size_t size, const spz::detail::BlockTable &t, int32_t to,
-                          SpzB200Cloud *out, int32_t *antialiased, void *stream, bool *taken) {
-  *taken = false;
-  std::vector<uint8_t> head;
-  if (!spz::detail::inflatePrefix(bytes, size, spz::detail::kContainerHeaderBytes, &head) || head.size() < spz::detail::kContainerHeaderBytes)
-    return SPZB200_OK;
-  spz::detail::Container c;
-  if (!spz::detail::parseContainer(head.data(), (size_t)t.totalSize, &c)) return SPZB200_OK;  // reads the 16 bytes and the size
-  if (out->num_points != c.numPoints || out->sh_degree != c.shDegree || c.numPoints == 0) return SPZB200_OK;
-  if (checkCloud(out, "spzb200_load_spz_device")) return SPZB200_OK;
-  if (cudaSetDevice(ctx->device) != cudaSuccess) return SPZB200_OK;
-  const cudaStream_t st = (cudaStream_t)stream;
-  // stream order -> struct order (positions, scales, rotations, alphas, colors, sh)
-  const int structOf[6] = {0, 3, 4, 1, 2, 5};
-  size_t aligned = 0;
-  for (int i = 0; i < 6; i++) aligned += alignUp(c.bytes[i], 16);
-  DeviceScratch scratch(st);
-  uint8_t *container = nullptr, *base = nullptr;
-  if (scratch.alloc(&container, (size_t)t.totalSize) != cudaSuccess || scratch.alloc(&base, aligned) != cudaSuccess) {
-    cudaGetLastError();
-    return SPZB200_OK;
-  }
-  bool vouched = false;
-  if (inflateDeviceBytes(ctx, bytes, t, container, scratch, &vouched) != SPZB200_OK || !vouched) return SPZB200_OK;
-  // From here on the call's result is this route's: the container is what the host route would inflate.
-  *taken = true;
-  if (antialiased) *antialiased = c.antialiased ? 1 : 0;
-  uint8_t *planes[6];
-  for (int i = 0; i < 6; i++) {  // plane offsets such as 16 + 9n are not aligned: move the planes
-    planes[structOf[i]] = base;
-    if (c.bytes[i]) CU(cudaMemcpyAsync(base, container + c.offset[i], c.bytes[i], cudaMemcpyDeviceToDevice, st));
-    base += alignUp(c.bytes[i], 16);
-  }
+// The packed planes of a parsed container whose planes sit at `planes` (struct order).
+SpzB200Packed packedOfContainer(const spz::detail::Container &c, uint8_t *const planes[6]) {
   SpzB200Packed in;
   std::memset(&in, 0, sizeof in);
   in.num_points = c.numPoints;
@@ -2340,10 +2511,153 @@ int loadSpzDeviceInflated(SpzB200Context *ctx, const uint8_t *bytes, size_t size
   in.version = c.half ? SPZB200_STREAM_V1 : c.smallestThree ? SPZB200_STREAM_V3 : SPZB200_STREAM_V2;
   in.positions = planes[0]; in.scales = planes[1]; in.rotations = planes[2];
   in.alphas = planes[3]; in.colors = planes[4]; in.sh = c.shDegree ? planes[5] : nullptr;
-  const int rc = spzb200_decode_device(ctx, &in, to, out, stream);
+  return in;
+}
+
+// stream order -> struct order (positions, scales, rotations, alphas, colors, sh)
+constexpr int kStructOf[6] = {0, 3, 4, 1, 2, 5};
+
+// load_spz_device's host route: inflate on the host (block-parallel where a table allows), validate, copy
+// each plane up and decode on the device.  Its verdict is the file's.  Synchronous.
+int loadSpzHostRoute(SpzB200Context *ctx, const char *who, const uint8_t *bytes, size_t size, int32_t to, SpzB200Cloud *out,
+                     int32_t *antialiased, cudaStream_t st) {
+  std::vector<uint8_t> container;
+  if (!spz::decompressGzippedParallel(bytes, size, spz::detail::inflateThreads(), &container))
+    return fail(SPZB200_ERR_INVALID, "%s: not a readable gzip member", who);
+  spz::detail::Container c;
+  if (!spz::detail::parseContainer(container.data(), container.size(), &c))
+    return fail(SPZB200_ERR_INVALID, "%s: not an .spz container (bad magic, version, degree or size)", who);
+  if (out->num_points != c.numPoints || out->sh_degree != c.shDegree)
+    return fail(SPZB200_ERR_INVALID, "%s: out holds %lld points of SH degree %d, the file %d of degree %d (spzb200_spz_info)", who,
+                (long long)out->num_points, out->sh_degree, c.numPoints, c.shDegree);
+  int rc = checkCloud(out, who);
+  if (rc) return rc;
+  if (antialiased) *antialiased = c.antialiased ? 1 : 0;
+  if (c.numPoints == 0) return SPZB200_OK;
+  CU(cudaSetDevice(ctx->device));
+  size_t aligned = 0;
+  for (int i = 0; i < 6; i++) aligned += alignUp(c.bytes[i], 16);
+  DeviceScratch scratch(st);
+  uint8_t *base = nullptr;
+  CU(scratch.alloc(&base, aligned));
+  uint8_t *planes[6];
+  for (int i = 0; i < 6; i++) {
+    planes[kStructOf[i]] = base;
+    if (c.bytes[i]) CU(cudaMemcpyAsync(base, container.data() + c.offset[i], c.bytes[i], cudaMemcpyHostToDevice, st));
+    base += alignUp(c.bytes[i], 16);
+  }
+  const SpzB200Packed in = packedOfContainer(c, planes);
+  rc = spzb200_decode_device(ctx, &in, to, out, st);
   if (rc) return rc;
   CU(cudaStreamSynchronize(st));
   return SPZB200_OK;
+}
+
+// A file of a load batch that may take the device route: a member with a block table of blocks under
+// kDeviceLoadMaxBlock whose header (inflated on the host, 16 bytes) agrees with its `out`.
+struct DeviceLoad {
+  int index;
+  spz::detail::BlockTable t;
+  spz::detail::Container c;
+};
+
+bool deviceLoadCandidate(const uint8_t *bytes, size_t size, const SpzB200Cloud *out, const char *who, DeviceLoad *d) {
+  if (!spz::detail::parseBlockTable(bytes, size, &d->t) || d->t.blockSize >= kDeviceLoadMaxBlock) return false;
+  std::vector<uint8_t> head;
+  if (!spz::detail::inflatePrefix(bytes, size, spz::detail::kContainerHeaderBytes, &head) || head.size() < spz::detail::kContainerHeaderBytes)
+    return false;
+  if (!spz::detail::parseContainer(head.data(), (size_t)d->t.totalSize, &d->c)) return false;  // reads the 16 bytes and the size
+  if (out->num_points != d->c.numPoints || out->sh_degree != d->c.shDegree || d->c.numPoints == 0) return false;
+  return checkCloud(out, who) == SPZB200_OK;
+}
+
+// load_spz_device of `count` files (DESIGN.md section 10c).  The device-route candidates are inflated in one
+// launch into containers at 16-byte-aligned places of one buffer; one move launch puts every vouched
+// container's planes at aligned places; each cloud is decoded by its own launches, queued with no host
+// wait in between.  Every other file, and every candidate the device cannot vouch for or whose device
+// scratch cannot be allocated, takes the host route alone.  status[i] is the file's verdict; a CUDA or
+// allocation failure outside the device route's own scratch ends the call.
+int loadBatch(SpzB200Context *ctx, const char *who, const uint8_t *const *bytes, const size_t *sizes, int32_t count, int32_t to,
+              SpzB200Cloud *out, int32_t *antialiased, int32_t *status, cudaStream_t st) {
+  return guarded(who, nullptr, nullptr, [&]() -> int {
+    std::vector<char> hostRoute(count, 1);
+    std::vector<DeviceLoad> dev;
+    for (int i = 0; i < count; i++) {
+      status[i] = SPZB200_OK;
+      DeviceLoad d;
+      d.index = i;
+      if (deviceLoadCandidate(bytes[i], sizes[i], &out[i], who, &d)) dev.push_back(std::move(d));
+    }
+    if (!dev.empty() && cudaSetDevice(ctx->device) == cudaSuccess) {
+      const int n = (int)dev.size();
+      std::vector<uint64_t> containerBytes(n), planeBytes(n), containerAt, planesAt;
+      for (int k = 0; k < n; k++) {
+        containerBytes[k] = dev[k].t.totalSize;
+        for (int p = 0; p < 6; p++) planeBytes[k] += alignUp(dev[k].c.bytes[p], 16);
+      }
+      spzb200::planAligned(containerBytes.data(), n, &containerAt);
+      spzb200::planAligned(planeBytes.data(), n, &planesAt);
+      DeviceScratch scratch(st);
+      uint8_t *containers = nullptr, *base = nullptr;
+      std::vector<char> vouched;
+      bool inflated = false;
+      if (scratch.alloc(&containers, containerAt[n]) == cudaSuccess && scratch.alloc(&base, planesAt[n]) == cudaSuccess) {
+        std::vector<InflateMember> members(n);
+        for (int k = 0; k < n; k++) members[k] = {bytes[dev[k].index], &dev[k].t, containers + containerAt[k]};
+        inflated = inflateDeviceBatch(ctx, members, scratch, &vouched) == SPZB200_OK;
+      }
+      if (!inflated) cudaGetLastError();
+      // From here on a vouched file's result is this route's: its container is what the host route would inflate.
+      std::vector<spzb200::MoveSpan> spans;
+      std::vector<SpzB200Packed> packed;
+      std::vector<int> decoded;
+      unsigned long long maxSpan = 0;
+      for (int k = 0; inflated && k < n; k++) {
+        if (!vouched[k]) continue;
+        const int i = dev[k].index;
+        const spz::detail::Container &c = dev[k].c;
+        hostRoute[i] = 0;
+        if (antialiased) antialiased[i] = c.antialiased ? 1 : 0;
+        uint8_t *planes[6], *p = base + planesAt[k];
+        for (int s = 0; s < 6; s++) {  // plane offsets such as 16 + 9n are not aligned: move the planes
+          planes[kStructOf[s]] = p;
+          if (c.bytes[s]) {
+            spans.push_back({(unsigned long long)(uintptr_t)(containers + containerAt[k] + c.offset[s]), (unsigned long long)(uintptr_t)p,
+                             c.bytes[s]});
+            maxSpan = std::max<unsigned long long>(maxSpan, c.bytes[s]);
+          }
+          p += alignUp(c.bytes[s], 16);
+        }
+        packed.push_back(packedOfContainer(c, planes));
+        decoded.push_back(i);
+      }
+      if (!spans.empty()) {
+        spzb200::MoveSpan *dSpans = nullptr;
+        int rc = uploadTable(spans, &dSpans, scratch);
+        if (rc) return rc;
+        int launches = 0;
+        CU(spzb200::launchMoveSpans(dSpans, (long long)spans.size(), maxSpan, st, &launches));
+        ctx->kernelLaunches += launches;
+        for (size_t k = 0; k < decoded.size(); k++) {
+          rc = spzb200_decode_device(ctx, &packed[k], to, &out[decoded[k]], st);
+          if (rc) return rc;
+        }
+        CU(cudaStreamSynchronize(st));
+      }
+    }
+    bool failed = false;
+    for (int i = 0; i < count; i++) {
+      if (!hostRoute[i]) continue;
+      const int rc = loadSpzHostRoute(ctx, who, bytes[i], sizes[i], to, &out[i], antialiased ? &antialiased[i] : nullptr, st);
+      if (rc == SPZB200_ERR_INVALID) {
+        status[i] = rc;
+        failed = true;
+      } else if (rc) {
+        return rc;
+      }
+    }
+    return failed ? SPZB200_ERR_INVALID : SPZB200_OK;
+  });
 }
 
 }  // namespace
@@ -2356,59 +2670,21 @@ int spzb200_load_spz_device(SpzB200Context *ctx, const uint8_t *bytes, size_t si
   if (!ctx) return fail(SPZB200_ERR_INVALID, "%s: null context", who);
   if (!bytes || !out) return fail(SPZB200_ERR_INVALID, "%s: null argument", who);
   if (to < 0 || to > 8) return fail(SPZB200_ERR_INVALID, "%s: coordinate system %d", who, to);
-  return guarded(who, nullptr, nullptr, [&]() -> int {
-    {
-      spz::detail::BlockTable t;
-      if (spz::detail::parseBlockTable(bytes, size, &t) && t.blockSize < kDeviceLoadMaxBlock) {
-        bool taken = false;
-        const int rc = loadSpzDeviceInflated(ctx, bytes, size, t, to, out, antialiased, stream, &taken);
-        if (taken) return rc;
-      }
-    }
-    // Members without a block table (the reference's files, small saveSpz files), with blocks of 1 MiB or
-    // more (saveSpz's zlib blocks), and those the device route could not finish: inflate on the host, copy
-    // the container's planes up, decode on the device.
-    std::vector<uint8_t> container;
-    if (!spz::decompressGzippedParallel(bytes, size, spz::detail::inflateThreads(), &container))
-      return fail(SPZB200_ERR_INVALID, "%s: not a readable gzip member", who);
-    spz::detail::Container c;
-    if (!spz::detail::parseContainer(container.data(), container.size(), &c))
-      return fail(SPZB200_ERR_INVALID, "%s: not an .spz container (bad magic, version, degree or size)", who);
-    if (out->num_points != c.numPoints || out->sh_degree != c.shDegree)
-      return fail(SPZB200_ERR_INVALID, "%s: out holds %lld points of SH degree %d, the file %d of degree %d (spzb200_spz_info)", who,
-                  (long long)out->num_points, out->sh_degree, c.numPoints, c.shDegree);
-    int rc = checkCloud(out, who);
-    if (rc) return rc;
-    if (antialiased) *antialiased = c.antialiased ? 1 : 0;
-    if (c.numPoints == 0) return SPZB200_OK;
-    CU(cudaSetDevice(ctx->device));
-    const cudaStream_t st = (cudaStream_t)stream;
-    // stream order -> struct order (positions, scales, rotations, alphas, colors, sh)
-    const int structOf[6] = {0, 3, 4, 1, 2, 5};
-    size_t aligned = 0;
-    for (int i = 0; i < 6; i++) aligned += alignUp(c.bytes[i], 16);
-    DeviceScratch scratch(st);
-    uint8_t *base = nullptr;
-    CU(scratch.alloc(&base, aligned));
-    uint8_t *planes[6];
-    for (int i = 0; i < 6; i++) {
-      planes[structOf[i]] = base;
-      if (c.bytes[i]) CU(cudaMemcpyAsync(base, container.data() + c.offset[i], c.bytes[i], cudaMemcpyHostToDevice, st));
-      base += alignUp(c.bytes[i], 16);
-    }
-    SpzB200Packed in;
-    std::memset(&in, 0, sizeof in);
-    in.num_points = c.numPoints;
-    in.sh_degree = c.shDegree;
-    in.fractional_bits = c.fractionalBits;
-    in.version = c.half ? SPZB200_STREAM_V1 : c.smallestThree ? SPZB200_STREAM_V3 : SPZB200_STREAM_V2;
-    in.positions = planes[0]; in.scales = planes[1]; in.rotations = planes[2];
-    in.alphas = planes[3]; in.colors = planes[4]; in.sh = c.shDegree ? planes[5] : nullptr;
-    rc = spzb200_decode_device(ctx, &in, to, out, stream);
-    if (rc) return rc;
-    CU(cudaStreamSynchronize(st));
-    return SPZB200_OK;
-  });
+  int32_t status = SPZB200_OK;
+  return loadBatch(ctx, who, &bytes, &size, 1, to, out, antialiased, &status, (cudaStream_t)stream);
+}
+
+int spzb200_load_spz_device_batch(SpzB200Context *ctx, const uint8_t *const *bytes, const size_t *sizes, int32_t count, int32_t to,
+                                  SpzB200Cloud *out, int32_t *antialiased, int32_t *status, void *stream) {
+  const char *who = "spzb200_load_spz_device_batch";
+  if (!ctx) return fail(SPZB200_ERR_INVALID, "%s: null context", who);
+  if (count < 0) return fail(SPZB200_ERR_INVALID, "%s: count %d", who, count);
+  if (to < 0 || to > 8) return fail(SPZB200_ERR_INVALID, "%s: coordinate system %d", who, to);
+  if (count == 0) return SPZB200_OK;
+  if (!bytes || !sizes || !out || !status) return fail(SPZB200_ERR_INVALID, "%s: null argument", who);
+  for (int i = 0; i < count; i++)
+    if (!bytes[i]) return fail(SPZB200_ERR_INVALID, "%s: null bytes[%d]", who, i);
+  return loadBatch(ctx, who, bytes, sizes, count, to, out, antialiased, status, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -150,23 +150,30 @@ cudaError_t divisionSelfCheck(int part, unsigned long long pairsPerThread, unsig
 // saturates bytes the way the kernels assume (decided once per context).  `scratch` = one device int.
 cudaError_t probePackCvt(cudaStream_t stream, int *scratch, int *ok);
 
-// Device deflater (deflate_kernels.cu, DESIGN.md section 10): `size` device bytes at src ->
-// dfl::segmentCount(size) coded segments in slots (deflateSlotBytes() each), their byte counts and
-// CRC-32s, offsets[0..segments] (offsets[segments] = body bytes) and the packed raw deflate body
-// (at most size + 16 bytes per segment).  Three launches, asynchronous on `stream`.
-size_t deflateSlotBytes();
-cudaError_t launchDeflate(const uint8_t *src, unsigned long long size, uint8_t *slots, uint32_t *segBytes, uint32_t *segCrc,
-                          unsigned long long *offsets, uint8_t *body, cudaStream_t stream, int *launches);
-// 16 bytes from the host argument list to device memory, stream-ordered (no pageable copy, no sync).
-cudaError_t launchStoreBytes16(uint8_t *dst, const uint8_t bytes[16], cudaStream_t stream);
+struct DeflateSegment;
+struct InflateBlock;
+struct MoveSpan;
 
-// Device inflater (inflate_kernels.cu, DESIGN.md section 10): table block i of a block-table gzip
-// member -- raw deflate bytes body[inOffset[i], inOffset[i + 1]) -- into out[i * blockSize, ...) (the
-// last block holds total - (blocks - 1) * blockSize bytes).  status[i] = ifl::kOk when the block filled
-// its slice exactly, crc[i] its CRC-32 then.  One launch, asynchronous on `stream`; *warpsPerCta is
-// the geometry chosen for the block count and SM count.
-cudaError_t launchInflate(const uint8_t *body, const unsigned long long *inOffset, long long blocks, unsigned long long blockSize,
-                          unsigned long long total, uint8_t *out, uint32_t *crc, int32_t *status, int smCount, cudaStream_t stream,
-                          int *warpsPerCta);
+// Device deflater (deflate_kernels.cu, DESIGN.md sections 10 and 10c): the `segments` segments of one or
+// more inputs (DeflateSegment descriptors on the device, batch_plan.hpp: planDeflate) -> coded segments in
+// slots (deflateSlotBytes() each), their byte counts and CRC-32s, offsets[0..segments] (the exclusive scan
+// of the byte counts; offsets[segments] = body bytes) and the packed raw deflate body, each input's
+// segments at a contiguous range (at most its size + 16 bytes per segment).  Three launches,
+// asynchronous on `stream`.
+size_t deflateSlotBytes();
+cudaError_t launchDeflate(const DeflateSegment *segs, unsigned long long segments, uint8_t *slots, uint32_t *segBytes, uint32_t *segCrc,
+                          unsigned long long *offsets, uint8_t *body, cudaStream_t stream, int *launches);
+
+// Device inflater (inflate_kernels.cu, DESIGN.md sections 10 and 10c): `blocks` table blocks of one or
+// more block-table gzip members (InflateBlock descriptors on the device, batch_plan.hpp: planInflate),
+// block i's raw deflate bytes at body + desc[i].in into its slice desc[i].out.  status[i] = ifl::kOk when
+// the block filled its slice exactly, crc[i] its CRC-32 then.  One launch (blocks > 0), asynchronous on
+// `stream`; *warpsPerCta is the geometry chosen for the batch's block count and the SM count.
+cudaError_t launchInflate(const uint8_t *body, const InflateBlock *desc, long long blocks, uint32_t *crc, int32_t *status, int smCount,
+                          cudaStream_t stream, int *warpsPerCta);
+
+// Device-to-device copies of `count` MoveSpan descriptors (on the device) in one launch (move_kernels.cu);
+// maxBytes = the largest span.  None for count = 0.
+cudaError_t launchMoveSpans(const MoveSpan *spans, long long count, unsigned long long maxBytes, cudaStream_t stream, int *launches);
 
 }  // namespace spzb200

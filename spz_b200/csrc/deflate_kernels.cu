@@ -1,17 +1,21 @@
-// Device deflater: device bytes -> raw deflate segments -> one contiguous body (DESIGN.md section 10).
+// Device deflater: device inputs -> raw deflate segments -> one contiguous body (DESIGN.md sections 10
+// and 10c).
 //
-// One CTA per 64 KiB segment.  The segment is staged in shared memory with one bulk async copy; the
+// One CTA per 64 KiB segment; a DeflateSegment descriptor names its bytes and whether it ends its input,
+// so the segments of many inputs are coded in one launch.  The segment is staged in shared memory with one bulk async copy; the
 // symbols (literals, distance-1 matches for runs) are found by every thread for its 128-byte slice --
 // a run crossing slices belongs to the slice it starts in, whose thread learns its full length from a
 // CTA-wide pointer-jumping pass over the slices' head runs.  A histogram, the length-limited code
 // (package-merge, per-item steps spread over the threads), the header (one thread), a scan of the
 // threads' bit counts and an OR-assembly of the codes into shared words follow; the coded segment (or
 // its stored form, when that is not larger) goes to the segment's worst-case slot.  A second kernel
-// scans the segment sizes and a third packs the slots into one body.  All format decisions live in
+// scans the segment sizes of the whole batch and a third packs the slots into one body, each input's
+// segments at a contiguous range of it.  All format decisions live in
 // deflate_format.cuh, which tests compile for the host.
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "batch_plan.hpp"
 #include "codec_kernels.cuh"
 #include "deflate_format.cuh"
 #include "kernel_utils.cuh"
@@ -46,19 +50,19 @@ struct DeflateSmem {
 };
 
 __global__ void __launch_bounds__(kThreads, 1)
-    deflateSegmentsKernel(const uint8_t *__restrict__ src, unsigned long long size, unsigned long long segments,
-                          uint8_t *__restrict__ slots, uint32_t *__restrict__ segBytes, uint32_t *__restrict__ segCrc, int bulk) {
+    deflateSegmentsKernel(const DeflateSegment *__restrict__ desc, uint8_t *__restrict__ slots, uint32_t *__restrict__ segBytes,
+                          uint32_t *__restrict__ segCrc) {
   extern __shared__ __align__(16) uint8_t smemRaw[];
   DeflateSmem &S = *reinterpret_cast<DeflateSmem *>(smemRaw);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const unsigned long long seg = blockIdx.x;
-  const unsigned long long off = seg * kSegBytes;
-  const int len = (int)(size - off < (unsigned long long)kSegBytes ? size - off : kSegBytes);
-  const bool last = seg + 1 == segments;
-  const uint8_t *g = src + off;
+  const DeflateSegment d = desc[seg];
+  const int len = (int)d.len;
+  const bool last = d.last != 0;
+  const uint8_t *g = reinterpret_cast<const uint8_t *>(d.src);
 
   // ---- stage the segment; clear the output words and the histogram --------------------------------
-  const int bulkBytes = bulk ? (len & ~15) : 0;
+  const int bulkBytes = (d.src & 15) == 0 ? (len & ~15) : 0;
   if (tid == 0 && bulkBytes) {
     mbarInit(&S.bar);
     bulkLoad(S.in, g, (uint32_t)bulkBytes, &S.bar);
@@ -292,34 +296,18 @@ __global__ void __launch_bounds__(256)
   }
 }
 
-struct Header16 {
-  uint8_t b[16];
-};
-__global__ void storeBytesKernel(uint8_t *dst, Header16 h) {
-  if (threadIdx.x < 16) dst[threadIdx.x] = h.b[threadIdx.x];
-}
-
 }  // namespace
 
 size_t deflateSlotBytes() { return kSlotBytes; }
 
-cudaError_t launchDeflate(const uint8_t *src, unsigned long long size, uint8_t *slots, uint32_t *segBytes, uint32_t *segCrc,
+cudaError_t launchDeflate(const DeflateSegment *segs, unsigned long long segments, uint8_t *slots, uint32_t *segBytes, uint32_t *segCrc,
                           unsigned long long *offsets, uint8_t *body, cudaStream_t stream, int *launches) {
-  const unsigned long long segments = segmentCount(size);
   cudaError_t e = cudaFuncSetAttribute(deflateSegmentsKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(DeflateSmem));
   if (e != cudaSuccess) return e;
-  const int bulk = ((uintptr_t)src & 15) == 0;
-  deflateSegmentsKernel<<<(unsigned)segments, kThreads, sizeof(DeflateSmem), stream>>>(src, size, segments, slots, segBytes, segCrc, bulk);
+  deflateSegmentsKernel<<<(unsigned)segments, kThreads, sizeof(DeflateSmem), stream>>>(segs, slots, segBytes, segCrc);
   segmentOffsetsKernel<<<1, kScanThreads, 0, stream>>>(segBytes, segments, offsets);
   packSlotsKernel<<<(unsigned)segments, 256, 0, stream>>>(slots, segBytes, offsets, body);
   *launches = 3;
-  return cudaGetLastError();
-}
-
-cudaError_t launchStoreBytes16(uint8_t *dst, const uint8_t bytes[16], cudaStream_t stream) {
-  Header16 h;
-  for (int i = 0; i < 16; i++) h.b[i] = bytes[i];
-  storeBytesKernel<<<1, 32, 0, stream>>>(dst, h);
   return cudaGetLastError();
 }
 

@@ -1,7 +1,8 @@
-// Device inflater: the table blocks of a block-table gzip member -> their slices of the output
-// (DESIGN.md section 10).
+// Device inflater: the table blocks of block-table gzip members -> their slices of the outputs
+// (DESIGN.md sections 10 and 10c).
 //
-// One warp per table block.  The warp's lanes run inflate_format.cuh's decoder in lockstep on identical
+// One warp per table block; an InflateBlock descriptor names the block's compressed bytes and its output
+// slice, so the blocks of many members, each with its own block size, go to their own outputs in one launch.  The warp's lanes run inflate_format.cuh's decoder in lockstep on identical
 // state (no shuffles: they read the same bits and the same shared table entries); the code tables are
 // filled lane-parallel in the warp's shared workspace, lane 0 writes literals, and match and stored
 // copies are spread over the lanes.  Output goes straight to the block's slice in global memory,
@@ -11,6 +12,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "batch_plan.hpp"
 #include "codec_kernels.cuh"
 #include "deflate_format.cuh"
 #include "inflate_format.cuh"
@@ -40,9 +42,8 @@ __device__ __forceinline__ uint32_t crcBytes(const uint32_t *tab, uint32_t c, co
 }
 
 __global__ void __launch_bounds__(kMaxWarps * 32)
-    inflateBlocksKernel(const uint8_t *__restrict__ body, const unsigned long long *__restrict__ inOffset, long long blocks,
-                        unsigned long long blockSize, unsigned long long total, uint8_t *out, uint32_t *__restrict__ crcOut,
-                        int32_t *__restrict__ status) {
+    inflateBlocksKernel(const uint8_t *__restrict__ body, const InflateBlock *__restrict__ desc, long long blocks,
+                        uint32_t *__restrict__ crcOut, int32_t *__restrict__ status) {
   extern __shared__ __align__(16) uint8_t smemRaw[];
   uint32_t *crcTab = reinterpret_cast<uint32_t *>(smemRaw);
   ifl::Workspace *ws = reinterpret_cast<ifl::Workspace *>(smemRaw + 256 * sizeof(uint32_t)) + (threadIdx.x >> 5);
@@ -51,10 +52,10 @@ __global__ void __launch_bounds__(kMaxWarps * 32)
   const int lane = threadIdx.x & 31;
   const long long b = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (b >= blocks) return;
-  const unsigned long long start = (unsigned long long)b * blockSize;
-  const uint32_t len = (uint32_t)(b + 1 == blocks ? total - start : blockSize);
-  uint8_t *slice = out + start;
-  const int st = ifl::inflateBlock(body + inOffset[b], inOffset[b + 1] - inOffset[b], slice, len, ws, lane, 32, WarpSync{});
+  const InflateBlock d = desc[b];
+  const uint32_t len = d.outBytes;
+  uint8_t *slice = reinterpret_cast<uint8_t *>(d.out);
+  const int st = ifl::inflateBlock(body + d.in, d.inBytes, slice, len, ws, lane, 32, WarpSync{});
   if (st != ifl::kOk) {
     if (lane == 0) status[b] = st;
     return;
@@ -81,10 +82,9 @@ __global__ void __launch_bounds__(kMaxWarps * 32)
 
 }  // namespace
 
-cudaError_t launchInflate(const uint8_t *body, const unsigned long long *inOffset, long long blocks, unsigned long long blockSize,
-                          unsigned long long total, uint8_t *out, uint32_t *crc, int32_t *status, int smCount, cudaStream_t stream,
-                          int *warpsPerCta) {
-  // Each block is one serial decode, so the block count bounds the parallelism: with fewer than
+cudaError_t launchInflate(const uint8_t *body, const InflateBlock *blocksDesc, long long blocks, uint32_t *crc, int32_t *status, int smCount,
+                          cudaStream_t stream, int *warpsPerCta) {
+  // Each block is one serial decode, so the block count of the whole batch bounds the parallelism: with fewer than
   // kMaxWarps blocks per SM (1 MiB zlib blocks: 620 for a 10M SH3 file) every warp gets a CTA of its
   // own so the blocks spread over all SMs; otherwise kMaxWarps warps share a CTA and its CRC table.
   const int warps = blocks >= (long long)kMaxWarps * (smCount > 0 ? smCount : 1) ? kMaxWarps : 1;
@@ -93,7 +93,7 @@ cudaError_t launchInflate(const uint8_t *body, const unsigned long long *inOffse
   cudaError_t e = cudaFuncSetAttribute(inflateBlocksKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   const long long ctas = (blocks + warps - 1) / warps;
-  inflateBlocksKernel<<<(unsigned)ctas, warps * 32, smem, stream>>>(body, inOffset, blocks, blockSize, total, out, crc, status);
+  inflateBlocksKernel<<<(unsigned)ctas, warps * 32, smem, stream>>>(body, blocksDesc, blocks, crc, status);
   return cudaGetLastError();
 }
 
